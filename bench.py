@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py -- GDoF/s of the matrix-free multigrid hot path on B200 (contract: see task prompt 4).
+"""bench.py -- GDoF/s of the matrix-free multigrid hot path on B200.
 
 A step = one V-cycle (VCycleMultigrid::vmult, reference include/multigrid/portable_v_cycle_multigrid.h:79-94)
 on BASELINE.json configs[1]: 3-D Poisson, Q4, 64^3 cells (16 974 593 DoFs), polynomial multigrid
@@ -9,17 +9,25 @@ HBM.  `e2e` = the same through the C-ABI's host-buffer entry (pmg_vcycle_vmult_h
 from pinned memory, V-cycle, D2H of the correction).  `roofline` = the dominant kernel (the fused
 Chebyshev step on the finest level) timed alone with CUDA events on the library's stream.
 `--impl reference` times the reference's CPU algorithm (the oracle port: the reference itself cannot be
-compiled here) on the host cores for the same metric and the same workload (the configuration's one-GPU mesh; the sample
-is bounded by the number of cycles: <= 1 warm-up + <= 2 timed).
+compiled here) on the host cores for the same metric and the same workload (the configuration's one-GPU mesh; by default
+1 warm-up + 2 timed cycles, since one takes seconds).
+`--dump-outputs DIR` writes the GPU V-cycle's output of the last timed step to DIR/vcycle_z.npy (float64; above DUMP_MAX
+DoFs a fixed, seeded sample of them), so that two builds can be compared output for output on identical inputs.
+The bench writes nothing into the source tree (it may be read-only): no bytecode, and the oracle for the CPU legs is
+compiled into a temporary directory.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+import numpy as np
+
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "portable-multigrid_b200", "python"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -28,6 +36,10 @@ METRIC = "GDoF/s of one multigrid V-cycle (fine-level DoFs / time); operator-app
 UNIT = "GDoF/s"
 DEGREE = 4
 CELLS = 64
+GPU_STEPS, GPU_WARMUP = 50, 5
+REFERENCE_STEPS, REFERENCE_WARMUP = 2, 1  # the CPU arm: ~10-20 s per V-cycle at the flagship size
+DUMP_MAX = 1 << 22  # values per dumped array: 32 MB of float64
+DUMP_SEED = 0
 
 
 def scaled_cells(n, world):
@@ -146,11 +158,34 @@ def ncu_traffic():
         return None
 
 
+def load_oracle():
+    """The oracle compiled into a temporary directory (the source tree may be read-only): -march=native, or, where that
+    does not compile, the portable build.  Returns (module, kind)."""
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import pyoracle as O
+
+    with tempfile.TemporaryDirectory() as tmp:  # the library is loaded before the directory goes
+        try:
+            O.use_library(O.build(native=True, out_dir=tmp))
+            return O, "port (-march=native)"
+        except Exception:
+            O.use_library(O.build(out_dir=tmp))
+            return O, "port"
+
+
+def dump_outputs(out_dir, name, v):
+    """DIR/<name>.npy: v as float64, or, above DUMP_MAX entries, its entries at DUMP_MAX fixed, seeded, sorted indices."""
+    if v.size > DUMP_MAX:
+        v = v[np.sort(np.random.default_rng(DUMP_SEED).choice(v.size, DUMP_MAX, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v, dtype=np.float64))
+
+
 def run_reference(args, cfg):
     """CPU arm: the oracle's V-cycle (port of the reference algorithm in the reference's data layout) on all host threads,
     on the SAME workload as the product arm at one GPU -- the configuration's own mesh and hierarchy (64^3 cells Q4 for c2:
-    3.7 GB of stored indices / Jacobians, ~10-20 s per V-cycle); the sample is bounded by the number of cycles (<= 1 warm-up,
-    <= 2 timed).  Under torchrun the product arm weak-scales the mesh; this arm keeps the one-GPU mesh (the CPU's throughput
+    3.7 GB of stored indices / Jacobians, ~10-20 s per V-cycle), so by default 1 warm-up and 2 timed cycles (REFERENCE_STEPS,
+    REFERENCE_WARMUP; --steps / --warmup as given otherwise).  Under torchrun the product arm weak-scales the mesh; this arm keeps the one-GPU mesh (the CPU's throughput
     does not depend on the size beyond its caches) and `config.workload` names what it ran."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -158,17 +193,9 @@ def run_reference(args, cfg):
     # torchrun exports OMP_NUM_THREADS=1 to its workers; this arm is meant to use all the host threads it can
     if "LOCAL_RANK" in os.environ or os.environ.get("OMP_NUM_THREADS") == "1":
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import pyoracle as O
-
-    try:
-        O.build(native=True)
-        O.use_native()
-        kind = "port (-march=native)"
-    except Exception:
-        kind = "port"
+    O, kind = load_oracle()
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    res = cpu_vcycle(O, cfg, steps=min(max(args.steps, 1), 2), warmup=min(args.warmup, 1))
+    res = cpu_vcycle(O, cfg, steps=args.steps, warmup=args.warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": res["steps"], "warmup": res["warmup"], "ms_per_step": res["ms_per_step"], "higher_is_better": True,
@@ -216,23 +243,39 @@ def cpu_vcycle(O, cfg, steps, warmup):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed V-cycles (default %d; %d with --impl reference)" % (GPU_STEPS, REFERENCE_STEPS))
+    ap.add_argument("--warmup", type=int, default=None,
+                    help="untimed V-cycles before them (default %d, at least 3 on the GPU: eager, capture, replay; "
+                         "%d with --impl reference)" % (GPU_WARMUP, REFERENCE_WARMUP))
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS), help="BASELINE.json workload (default: the one the metric is quoted on)")
     ap.add_argument("--degree", type=int, default=None)
     ap.add_argument("--cells", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the GPU V-cycle's output of the last timed step to DIR/vcycle_z.npy")
     args = ap.parse_args()
+    reference = args.impl == "reference"
+    if args.steps is None:
+        args.steps = REFERENCE_STEPS if reference else GPU_STEPS
+    if args.warmup is None:
+        args.warmup = REFERENCE_WARMUP if reference else GPU_WARMUP
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if reference and args.dump_outputs:
+        # the CPU arm runs its own residual (zero on Dirichlet DoFs): nothing it computes is comparable with a GPU dump
+        ap.error("--dump-outputs writes the GPU path's output; it does not apply to --impl reference")
     cfg = dict(CONFIGS[args.config])
     if args.degree is not None:
         cfg["degree"] = args.degree
     if args.cells is not None:
         cfg["cells"] = args.cells
-    if args.impl == "reference":
+    if reference:
         return run_reference(args, cfg)
 
-    import numpy as np
     import torch
     import pmg_b200 as G
     from helpers import splitmix_src
@@ -304,6 +347,11 @@ def main():
         sampler.start()
     ms = timed(lambda: mg.vmult(z, r), args.steps)
     value = n_dofs / (ms * 1e-3) / 1e9
+    if args.dump_outputs:
+        z_host = z.export_host()  # now: the measurements below reuse z; with several ranks a collective gather
+        if rank == 0:
+            dump_outputs(args.dump_outputs, "vcycle_z", z_host)
+        del z_host
 
     # operator apply alone (LaplaceOperator::vmult), and the dominant kernel of the cycle
     u, b, xo = top.vector_from(splitmix_src(n_dofs, salt=1)), top.vector_from(splitmix_src(n_dofs, salt=2)), top.initialize_dof_vector()
@@ -460,14 +508,7 @@ def main():
     }
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         try:
-            sys.path.insert(0, os.path.join(ROOT, "oracle"))
-            import pyoracle as O
-
-            try:
-                O.build(native=True)
-                O.use_native()
-            except Exception:
-                pass
+            O, _ = load_oracle()
             res = cpu_vcycle(O, cfg, steps=1, warmup=1)
             line["cpu_baseline"] = {"value": res["value"], "unit": UNIT, "cores": res["cores"], "kind": "port", "sample": res["sample"],
                                     "apply_gdofs": res["apply_gdofs"]}

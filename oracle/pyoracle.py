@@ -14,17 +14,20 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _dp = C.POINTER(C.c_double)
 
 
-def build(native=False):
-    """Compile the oracle (make). native=True builds -march=native into a second .so."""
-    args = ["make", "-C", _HERE] + (["native"] if native else [])
+def build(native=False, out_dir=None):
+    """Compile the oracle (make) into oracle/_build, or into out_dir (the source tree may be read-only).
+    native=True builds -march=native into a second .so."""
+    out = os.path.join(out_dir or os.path.join(_HERE, "_build"), "liborc_native.so" if native else "liborc.so")
+    args = ["make", "-C", _HERE, "OUT=" + out] + (["MARCH=native"] if native else [])
     subprocess.run(args, check=True, stdout=subprocess.DEVNULL)
-    return os.path.join(_HERE, "_build", "liborc_native.so" if native else "liborc.so")
+    return out
 
 
-def _load(native=False):
-    path = os.path.join(_HERE, "_build", "liborc_native.so" if native else "liborc.so")
-    if not os.path.exists(path):
-        path = build(native)
+def _load(native=False, path=None):
+    if path is None:
+        path = os.path.join(_HERE, "_build", "liborc_native.so" if native else "liborc.so")
+        if not os.path.exists(path):
+            path = build(native)
     lib = C.CDLL(path)
     vp = C.c_void_p
     lib.orc_mf_create.restype = vp
@@ -62,10 +65,10 @@ def lib():
     return _lib
 
 
-def use_native():
-    """Switch to the -march=native build (bench.py cpu_baseline on the GPU box's host)."""
+def use_library(path):
+    """Switch to the oracle library at `path`, as returned by build(native, out_dir) (bench.py's CPU legs)."""
     global _lib
-    _lib = _load(True)
+    _lib = _load(path=path)
 
 
 def _p(a):
