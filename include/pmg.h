@@ -84,6 +84,18 @@ int64_t pmg_context_fused_halo_count(const pmg_context *ctx);
    1 = a(x) = 1/(0.05 + 2|x|^2) at the quadrature points (BASELINE config 5 extension). */
 int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz,
                                 unsigned dirichlet_faces, int coefficient, pmg_operator **op);
+/* The Laplace operator (with coefficient 0 or 1 as above) on a deformed structured hexahedral mesh of nx x ny x nz cells, 3-D
+   only.  vertices: HOST array of the (nx+1)(ny+1)(nz+1) mesh vertices, (x, y, z) interleaved, in global lexicographic order
+   (x fastest), the same full array on every rank; it is read during the call only.  Cell (cx, cy, cz) is the trilinear map
+   of its 8 vertices (cx+i, cy+j, cz+k), i, j, k in {0, 1} -- the geometry MappingQ(p) gives such a mesh with deal.II's
+   FlatManifold.  DoF numbering and Dirichlet faces are those of pmg_laplace_operator_create; the coefficient is evaluated
+   at the mapped quadrature points.  Every other operator, transfer, smoother, V-cycle and CG entry takes the result;
+   assemble_rhs and solution_norm integrate over the mapped cells (QGauss(p+1) and QGauss(p+2)).  For the h-transfer the
+   coarse mesh's vertex (i, j, k) must be the fine mesh's vertex (2i, 2j, 2k) (nested meshes; not checked).
+   Errors: PMG_ERR_ARG with the first offending cell in pmg_last_error() if a cell has det J <= 0 at one of its Gauss points
+   (inverted or degenerate) or a vertex that is not finite; PMG_ERR_UNSUPPORTED for degrees outside 1..PMG_MAX_DEGREE. */
+int pmg_laplace_operator_create_mapped(pmg_context *ctx, int degree, int nx, int ny, int nz, unsigned dirichlet_faces,
+                                       int coefficient, const double *vertices, pmg_operator **op);
 int pmg_laplace_operator_destroy(pmg_operator *op);
 int pmg_laplace_operator_vmult(const pmg_operator *op, pmg_vector *dst, const pmg_vector *src);  /* :557-719 */
 int pmg_laplace_operator_Tvmult(const pmg_operator *op, pmg_vector *dst, const pmg_vector *src); /* :721-735 */

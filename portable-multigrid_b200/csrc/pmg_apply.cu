@@ -111,6 +111,9 @@ int pmg_dim2_apply(const pmgk_level *lv, int mode, const double *u, const double
 // variable-coefficient levels: csrc/pmg_apply_var.cu
 int pmg_var_dispatch(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out,
                      double f1, double f2, cudaStream_t s, int *geom);
+// levels with mapped geometry: csrc/pmg_apply_geo.cu
+int pmg_geo_dispatch(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out,
+                     double f1, double f2, cudaStream_t s, int *geom);
 
 /* Small coarse levels run the cell-tile kernel (direct loads, lowest launch-to-result latency on one GPU) -- unless the level is
    a slab with neighbours: there every apply of the cell-tile kernel costs a ghost exchange (~17-30 us), which the plane-per-step
@@ -132,6 +135,7 @@ static int dispatch(const pmgk_level *lv, int mode, const double *u, const doubl
   if (part != PMGK_PART_ALL && !chunked_kernel) return PMG_ERR_UNSUPPORTED;
   if (lv->dim == 2) return pmg_dim2_apply(lv, mode, u, b, xold, out, f1, f2, s, geom);
   if (lv->nz < 1 || lv->cz_hi <= lv->cz_lo) return PMG_ERR_ARG;
+  if (lv->coef && lv->geo_stride) return pmg_geo_dispatch(lv, mode, u, b, xold, out, f1, f2, s, geom);
   if (lv->coef) return pmg_var_dispatch(lv, mode, u, b, xold, out, f1, f2, s, geom);
   /* tile_variant 0 (default): the line-marching kernel for levels large enough to fill its copy pipeline, the cell-tile
      kernel (direct loads, no staging prologue) for the small coarse levels, where launch-to-result latency is everything:

@@ -27,23 +27,6 @@ pmg_var_kernel(const __grid_constant__ PmgVarParams<P> p)
   Tile::run(p, ex, pmg_var_smem, tile_x, tile_y, chunk);
 }
 
-// number of z-chunks: minimise waves * (layers + recomputed layer below the chunk)
-void choose_var_chunks(int tiles, int layers, int slots, int *n_chunks, int *layers_per_chunk)
-{
-  long best_cost = -1;
-  int best_c = 1;
-  for (int c = 1; c <= layers; ++c) {
-    const int lpc = (layers + c - 1) / c;
-    const int used = (layers + lpc - 1) / lpc;
-    if (used != c) continue;
-    const long waves = ((long)tiles * c + slots - 1) / slots;
-    const long cost = waves * (lpc + (c > 1 ? 1 : 0));
-    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_c = c; }
-  }
-  *n_chunks = best_c;
-  *layers_per_chunk = (layers + best_c - 1) / best_c;
-}
-
 template <int P, int BX, int BY, int MINB>
 int launch_var(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out,
                double f1, double f2, cudaStream_t stream, int *geom)
@@ -74,7 +57,7 @@ int launch_var(const pmgk_level *lv, int mode, const double *u, const double *b,
     __atomic_store_n(&ctas_per_sm_dev[dev], ctas_per_sm, __ATOMIC_RELEASE);
   }
   const int slots = pmgk_device_sm_count() * ctas_per_sm;
-  choose_var_chunks(p.tiles_x * p.tiles_y, lv->cz_hi - lv->cz_lo, slots, &p.n_chunks, &p.layers_per_chunk);
+  pmg_var_choose_chunks(p.tiles_x * p.tiles_y, lv->cz_hi - lv->cz_lo, slots, &p.n_chunks, &p.layers_per_chunk);
   for (int i = 0; i < N1 * N1; ++i) { p.S[i] = lv->Sq[i]; p.D[i] = lv->Dco[i]; }
   for (int i = 0; i < N1; ++i) p.lam[i] = 0.0;
   p.c[0] = lv->h[1] * lv->h[2] / lv->h[0];
@@ -130,8 +113,6 @@ __global__ void k_var_dinv(const __grid_constant__ VarTables t, int nx, int ny, 
   }
 }
 
-int row_threads(int n) { return n >= 192 ? 256 : (n >= 96 ? 128 : (n >= 48 ? 64 : 32)); }
-
 template <int P>
 int fill_coef(const pmgk_level *lv, const double *gq, const double *gw, double *coef, cudaStream_t s)
 {
@@ -144,7 +125,7 @@ int fill_coef(const pmgk_level *lv, const double *gq, const double *gw, double *
   int64_t rows = (int64_t)Qy * nqz;
   const int64_t cap = (int64_t)pmgk_device_sm_count() * 32;
   if (rows > cap) rows = cap;
-  k_var_coef<P><<<(unsigned)rows, row_threads(Qx), 0, s>>>(t, Qx, Qy, lv->coef_cz0 * N1, nqz, coef);
+  k_var_coef<P><<<(unsigned)rows, pmg_var_row_threads(Qx), 0, s>>>(t, Qx, Qy, lv->coef_cz0 * N1, nqz, coef);
   PMG_CUDA_CHECK(cudaGetLastError());
   pmg_count_launch(1);
   return 0;
@@ -164,7 +145,7 @@ int fill_dinv(const pmgk_level *lv, const double *S2, const double *G2, double *
   int64_t rows = (int64_t)lv->Ny * lv->nzl;
   const int64_t cap = (int64_t)pmgk_device_sm_count() * 32;
   if (rows > cap) rows = cap;
-  k_var_dinv<P><<<(unsigned)rows, row_threads(lv->Nx), 0, s>>>(t, lv->nx, lv->ny, lv->Nx, lv->Ny, lv->Nz, lv->z0, lv->nzl,
+  k_var_dinv<P><<<(unsigned)rows, pmg_var_row_threads(lv->Nx), 0, s>>>(t, lv->nx, lv->ny, lv->Nx, lv->Ny, lv->Nz, lv->z0, lv->nzl,
                                                                lv->coef_cz0, lv->cz_hi, lv->faces, lv->coef, lv->coef_cz0, dinv);
   PMG_CUDA_CHECK(cudaGetLastError());
   pmg_count_launch(1);

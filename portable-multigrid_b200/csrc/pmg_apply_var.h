@@ -25,6 +25,7 @@
 //
 // Written against the same executor as the other tile programs: runs under tests/emu on the CPU test-suite.
 #pragma once
+#include <type_traits>
 #include "pmg_apply_tile.h"
 
 template <int P>
@@ -33,6 +34,13 @@ struct PmgVarParams : PmgApplyParams<P> {
   double D[(P + 1) * (P + 1)]; // co_shape_gradients D[q][r]: derivative of the Gauss-point Lagrange basis r at Gauss point q
   const double *coef;          // w_q a(x_q) on the lexicographic quadrature-point grid, cell layers from coef_cz0 on
   int coef_cz0;                // first cell layer stored in coef
+};
+
+// mapped geometry (PmgVarTile<.., GEO = true>): coef holds six quadrature-point grids, one per entry of the symmetric
+// G_q = w_q a(x(xi_q)) |det J_q| J_q^-1 J_q^-T  in the order xx, xy, xz, yy, yz, zz, grid k at coef + k * gstride
+template <int P>
+struct PmgGeoParams : PmgVarParams<P> {
+  int64_t gstride;
 };
 
 // the C5 coefficient a(x) = 1 / (0.05 + 2 |x|^2) (oracle/mesh.c: orc_coef_c5) times the quadrature weight, at
@@ -85,6 +93,98 @@ PMG_HD double pmg_var_diag_entry(int gx, int gy, int gz, int nx, int ny, int cz_
   return diag;
 }
 
+// diagonal entry of the mapped operator: sum over the <= 8 cells that contain dof (gx, gy, gz) of
+//   sum_q sum_{d,e} G_de(q) d_d phi_i(q) d_e phi_i(q),   d_x phi_i = G(qx,ix) S(qy,iy) S(qz,iz) etc.;
+// S2 / G2 as above, SG[q][i] = S(q,i) G(q,i) for the cross terms; geo: the six grids of PmgGeoParams, gstride apart
+template <int P>
+PMG_HD double pmg_geo_diag_entry(int gx, int gy, int gz, int nx, int ny, int cz_min, int cz_max, const double *S2,
+                                 const double *G2, const double *SG, const double *geo, int64_t gstride, int coef_cz0)
+{
+  constexpr int N1 = P + 1;
+  const int Qx = nx * N1;
+  const int64_t Qplane = (int64_t)Qx * (ny * N1);
+  double diag = 0.0;
+  for (int ez = 0; ez < 2; ++ez) {
+    const int cz = gz / P - ez, iz = gz - cz * P;
+    if (cz < cz_min || cz >= cz_max || iz > P) continue;
+    for (int ey = 0; ey < 2; ++ey) {
+      const int cy = gy / P - ey, iy = gy - cy * P;
+      if (cy < 0 || cy >= ny || iy > P) continue;
+      for (int ex = 0; ex < 2; ++ex) {
+        const int cx = gx / P - ex, ix = gx - cx * P;
+        if (cx < 0 || cx >= nx || ix > P) continue;
+        const double *cw = geo + (int64_t)(cz - coef_cz0) * N1 * Qplane + (int64_t)(cy * N1) * Qx + cx * N1;
+        for (int m = 0; m < N1; ++m) {
+          const double sz = S2[m * N1 + iz], dz = G2[m * N1 + iz], xz = SG[m * N1 + iz];
+          for (int b = 0; b < N1; ++b) {
+            const double sy = S2[b * N1 + iy], dy = G2[b * N1 + iy], xy = SG[b * N1 + iy];
+            const double *row = cw + m * Qplane + (int64_t)b * Qx;
+            double s = 0.0;
+            for (int a = 0; a < N1; ++a) {
+              const double sx = S2[a * N1 + ix], dx = G2[a * N1 + ix], xx = SG[a * N1 + ix];
+              s += row[a] * dx * sy * sz + row[3 * gstride + a] * sx * dy * sz + row[5 * gstride + a] * sx * sy * dz +
+                   2.0 * (row[gstride + a] * xx * xy * sz + row[2 * gstride + a] * xx * sy * xz + row[4 * gstride + a] * sx * xy * xz);
+            }
+            diag += s;
+          }
+        }
+      }
+    }
+  }
+  return diag;
+}
+
+// G_q of one quadrature point of the trilinear map of a cell: v[c][d] = coordinate d of the cell's vertex
+// c = ix + 2 iy + 4 iz; (xq, yq, zq) = the point on the reference cell [0,1]^3; wq = quadrature weight.  Writes the
+// six entries (xx, xy, xz, yy, yz, zz) of  wq a(x) |det J| J^-1 J^-T  (a = C5 coefficient at the mapped point when
+// c5 != 0, else 1) and returns det J (<= 0 or NaN: the cell is inverted or degenerate)
+PMG_HD double pmg_geo_point(const double (*v)[3], double xq, double yq, double zq, double wq, int c5, double *G)
+{
+  const double L[2][3] = {{1.0 - xq, 1.0 - yq, 1.0 - zq}, {xq, yq, zq}};
+  double J[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}}, x[3] = {0, 0, 0}; // J[d][e] = d x_d / d xi_e
+  for (int c = 0; c < 8; ++c) {
+    const int i = c & 1, j = c >> 1 & 1, k = c >> 2;
+    const double w = L[i][0] * L[j][1] * L[k][2];
+    const double d0 = (i ? 1.0 : -1.0) * L[j][1] * L[k][2], d1 = L[i][0] * (j ? 1.0 : -1.0) * L[k][2], d2 = L[i][0] * L[j][1] * (k ? 1.0 : -1.0);
+    for (int d = 0; d < 3; ++d) { x[d] += w * v[c][d]; J[d][0] += d0 * v[c][d]; J[d][1] += d1 * v[c][d]; J[d][2] += d2 * v[c][d]; }
+  }
+  // adjugate: J^-1 = adj(J) / det
+  const double A00 = J[1][1] * J[2][2] - J[1][2] * J[2][1], A01 = J[0][2] * J[2][1] - J[0][1] * J[2][2], A02 = J[0][1] * J[1][2] - J[0][2] * J[1][1];
+  const double A10 = J[1][2] * J[2][0] - J[1][0] * J[2][2], A11 = J[0][0] * J[2][2] - J[0][2] * J[2][0], A12 = J[0][2] * J[1][0] - J[0][0] * J[1][2];
+  const double A20 = J[1][0] * J[2][1] - J[1][1] * J[2][0], A21 = J[0][1] * J[2][0] - J[0][0] * J[2][1], A22 = J[0][0] * J[1][1] - J[0][1] * J[1][0];
+  const double det = J[0][0] * A00 + J[0][1] * A10 + J[0][2] * A20;
+  double f = wq / det; // w |det J| (adj/det)(adj/det)^T = w / det * adj adj^T for det > 0
+  if (c5) f *= 1.0 / (0.05 + 2.0 * (x[0] * x[0] + x[1] * x[1] + x[2] * x[2]));
+  G[0] = f * (A00 * A00 + A01 * A01 + A02 * A02);
+  G[1] = f * (A00 * A10 + A01 * A11 + A02 * A12);
+  G[2] = f * (A00 * A20 + A01 * A21 + A02 * A22);
+  G[3] = f * (A10 * A10 + A11 * A11 + A12 * A12);
+  G[4] = f * (A10 * A20 + A11 * A21 + A12 * A22);
+  G[5] = f * (A20 * A20 + A21 * A21 + A22 * A22);
+  return det;
+}
+
+// host side of the launchers (pmg_apply_var.cu, pmg_apply_geo.cu): number of z-chunks that minimises
+// waves * (layers + recomputed layer below the chunk)
+inline void pmg_var_choose_chunks(int tiles, int layers, int slots, int *n_chunks, int *layers_per_chunk)
+{
+  long best_cost = -1;
+  int best_c = 1;
+  for (int c = 1; c <= layers; ++c) {
+    const int lpc = (layers + c - 1) / c;
+    const int used = (layers + lpc - 1) / lpc;
+    if (used != c) continue;
+    const long waves = ((long)tiles * c + slots - 1) / slots;
+    const long cost = waves * (lpc + (c > 1 ? 1 : 0));
+    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_c = c; }
+  }
+  *n_chunks = best_c;
+  *layers_per_chunk = (layers + best_c - 1) / best_c;
+}
+
+// threads per CTA of the set-up kernels that walk one row of n points
+inline int pmg_var_row_threads(int n) { return n >= 192 ? 256 : (n >= 96 ? 128 : (n >= 48 ? 64 : 32)); }
+
 // hint: bring the line at `ptr` closer (L2, or L1 with PMG_VAR_PREFETCH_L1); the kernel's global loads are consumed right
 // where they are issued, two to three barriers after the place where their addresses are known
 PMG_HD void pmg_var_prefetch(const double *ptr)
@@ -100,9 +200,10 @@ PMG_HD void pmg_var_prefetch(const double *ptr)
 #endif
 }
 
-template <int P, int BX, int BY>
+template <int P, int BX, int BY, bool GEO = false>
 struct PmgVarTile {
   using Base = PmgApplyTile<P, BX, BY>;
+  using Params = std::conditional_t<GEO, PmgGeoParams<P>, PmgVarParams<P>>;
   using ThreadState = typename Base::ThreadState;
   static constexpr int N1 = Base::N1, CXC = Base::CXC, NITEM = Base::NITEM, NT = Base::NT, AP = Base::AP;
   static constexpr int T1_SIZE = Base::T1_SIZE, O_SIZE = Base::O_SIZE;
@@ -115,7 +216,7 @@ struct PmgVarTile {
   static constexpr int MSTRIDE = NITEM * AP; // distance between consecutive m
 
   // decode of the (cell, a) items of the y phases (as PmgApplyTile::phase_y): false = nothing to do
-  static PMG_HD bool decode_y(const PmgVarParams<P> &p, int tid, int cx0, int cy0, int &a, int &tcx, int &tcy)
+  static PMG_HD bool decode_y(const Params &p, int tid, int cx0, int cy0, int &a, int &tcx, int &tcy)
   {
     if (tid >= NITEM) return false;
     if (Base::Y_A_FASTEST) { a = tid % N1; tcx = (tid / N1) % CXC; tcy = tid / (N1 * CXC); }
@@ -125,7 +226,7 @@ struct PmgVarTile {
   }
 
   // Y1: values at the quadrature points (in place) and their y derivative (-> T2)
-  static PMG_HD void phase_y1(const PmgVarParams<P> &p, int tid, int cx0, int cy0, double *smem)
+  static PMG_HD void phase_y1(const Params &p, int tid, int cx0, int cy0, double *smem)
   {
     int a, tcx, tcy;
     if (!decode_y(p, tid, cx0, cy0, a, tcx, tcy)) return;
@@ -155,7 +256,7 @@ struct PmgVarTile {
   }
 
   // XZ: x and z derivative parts in registers, in place; the y derivative in T2 is scaled with its coefficient
-  static PMG_HD void phase_xz(const PmgVarParams<P> &p, const ThreadState &st, double *smem, int cz)
+  static PMG_HD void phase_xz(const Params &p, const ThreadState &st, double *smem, int cz)
   {
     if (!st.valid) return;
     double *t1 = smem + Base::t1_index(Base::item_index(st.tcx, st.j, st.tcy), 0, 0);
@@ -247,8 +348,66 @@ struct PmgVarTile {
       for (int a = 0; a < N1; ++a) t1[m * MSTRIDE + a] = R[m][a];
   }
 
+  // XZ of the mapped operator: all three reference derivatives of the points (a, b, m) meet in this thread -- x and z in
+  // registers, y in T2 -- so  (Gx, Gy, Gz) = G_q (gx, gy, gz)  is formed here; Gy goes back to T2 for Y2
+  static PMG_HD void phase_xz_geo(const Params &p, const ThreadState &st, double *smem, int cz)
+  {
+    if (!st.valid) return;
+    double *t1 = smem + Base::t1_index(Base::item_index(st.tcx, st.j, st.tcy), 0, 0);
+    double *t2 = t1 + T2_OFFSET;
+    const int Qx = p.nx * N1;
+    const int64_t Qplane = (int64_t)Qx * (p.ny * N1);
+    const double *cw = p.coef + (int64_t)(cz - p.coef_cz0) * N1 * Qplane + (int64_t)(st.cy * N1 + st.j) * Qx + st.cx * N1;
+    double R[N1][N1];
+#pragma unroll
+    for (int m = 0; m < N1; ++m)
+#pragma unroll
+      for (int a = 0; a < N1; ++a) R[m][a] = 0.0;
+#pragma unroll
+    for (int m = 0; m < N1; ++m) {
+      double gx[N1], gz[N1], Um[N1];
+#pragma unroll
+      for (int a = 0; a < N1; ++a) { Um[a] = t1[m * MSTRIDE + a]; gz[a] = 0.0; }
+#pragma unroll
+      for (int r = 0; r < N1; ++r) {
+#pragma unroll
+        for (int a = 0; a < N1; ++a) gz[a] += p.D[m * N1 + r] * t1[r * MSTRIDE + a];
+      }
+#pragma unroll
+      for (int a = 0; a < N1; ++a) {
+        double sx = 0.0;
+#pragma unroll
+        for (int r = 0; r < N1; ++r) sx += p.D[a * N1 + r] * Um[r];
+        const double *g = cw + m * Qplane + a;
+        const double gy = t2[m * MSTRIDE + a];
+        const double gxx = g[0], gxy = g[p.gstride], gxz = g[2 * p.gstride];
+        const double gyy = g[3 * p.gstride], gyz = g[4 * p.gstride], gzz = g[5 * p.gstride];
+        const double sz = gz[a];
+        gx[a] = gxx * sx + gxy * gy + gxz * sz;
+        t2[m * MSTRIDE + a] = gxy * sx + gyy * gy + gyz * sz;
+        gz[a] = gxz * sx + gyz * gy + gzz * sz;
+      }
+      // transposed derivatives
+#pragma unroll
+      for (int r = 0; r < N1; ++r) {
+        double s = R[m][r];
+#pragma unroll
+        for (int a = 0; a < N1; ++a) s += p.D[a * N1 + r] * gx[a];
+        R[m][r] = s;
+      }
+#pragma unroll
+      for (int r = 0; r < N1; ++r)
+#pragma unroll
+        for (int a = 0; a < N1; ++a) R[r][a] += p.D[m * N1 + r] * gz[a];
+    }
+#pragma unroll
+    for (int m = 0; m < N1; ++m)
+#pragma unroll
+      for (int a = 0; a < N1; ++a) t1[m * MSTRIDE + a] = R[m][a];
+  }
+
   // Y2: add the y derivative part, then the transposed interpolation along y, in place in T1
-  static PMG_HD void phase_y2(const PmgVarParams<P> &p, int tid, int cx0, int cy0, double *smem)
+  static PMG_HD void phase_y2(const Params &p, int tid, int cx0, int cy0, double *smem)
   {
     int a, tcx, tcy;
     if (!decode_y(p, tid, cx0, cy0, a, tcx, tcy)) return;
@@ -278,16 +437,26 @@ struct PmgVarTile {
 
   // thread (cell, j): prefetch the coefficient rows phase XZ of layer cz will read and the u rows phase F of layer
   // cz + 1 will read (a row = P+1 consecutive doubles: one or two 32-byte sectors)
-  static PMG_HD void prefetch_layer(const PmgVarParams<P> &p, const ThreadState &st, int cz, bool next_u)
+  static PMG_HD void prefetch_layer(const Params &p, const ThreadState &st, int cz, bool next_u)
   {
     if (!st.valid) return;
     const int Qx = p.nx * N1;
     const int64_t Qplane = (int64_t)Qx * (p.ny * N1);
     const double *cw = p.coef + (int64_t)(cz - p.coef_cz0) * N1 * Qplane + (int64_t)(st.cy * N1 + st.j) * Qx + st.cx * N1;
+    if constexpr (GEO) {
 #pragma unroll
-    for (int m = 0; m < N1; ++m) {
-      pmg_var_prefetch(cw + m * Qplane);
-      if (N1 > 4) pmg_var_prefetch(cw + m * Qplane + P);
+      for (int k = 0; k < 6; ++k)
+#pragma unroll
+        for (int m = 0; m < N1; ++m) {
+          pmg_var_prefetch(cw + k * p.gstride + m * Qplane);
+          if (N1 > 4) pmg_var_prefetch(cw + k * p.gstride + m * Qplane + P);
+        }
+    } else {
+#pragma unroll
+      for (int m = 0; m < N1; ++m) {
+        pmg_var_prefetch(cw + m * Qplane);
+        if (N1 > 4) pmg_var_prefetch(cw + m * Qplane + P);
+      }
     }
     if (next_u) {
       const int64_t plane = (int64_t)p.Nx * p.Ny;
@@ -301,7 +470,7 @@ struct PmgVarTile {
   }
 
   template <class Exec>
-  static PMG_HD void run(const PmgVarParams<P> &p, Exec &ex, double *smem, int tile_x, int tile_y, int chunk)
+  static PMG_HD void run(const Params &p, Exec &ex, double *smem, int tile_x, int tile_y, int chunk)
   {
     const int cx0 = tile_x * BX, cy0 = tile_y * BY;
     const int cz_begin = p.cz_lo + chunk * p.layers_per_chunk;
@@ -327,7 +496,8 @@ struct PmgVarTile {
       ex.sync();
       ex.for_each_thread([&](int tid, ThreadState &) { phase_y1(p, tid, cx0, cy0, smem); });
       ex.sync();
-      ex.for_each_thread([&](int, ThreadState &st) { phase_xz(p, st, smem, cz); });
+      if constexpr (GEO) ex.for_each_thread([&](int, ThreadState &st) { phase_xz_geo(p, st, smem, cz); });
+      else ex.for_each_thread([&](int, ThreadState &st) { phase_xz(p, st, smem, cz); });
       ex.sync();
       ex.for_each_thread([&](int tid, ThreadState &) { phase_y2(p, tid, cx0, cy0, smem); });
       ex.sync();

@@ -92,14 +92,43 @@ static double arg_double(int argc, char **argv, const char *name, double def)
 
 /* options shared by both drivers: --coefficient 1 solves -div(a grad u) = 1, a = 1/(0.05 + 2|x|^2) (BASELINE config 5),
    --tol T the relative CG tolerance (reference 1e-12, config 5: 1e-10), --profile 1 prints the per-level device time of one
-   V-cycle (smoother / transfer / halo / other) */
+   V-cycle (smoother / transfer / halo / other), --distort EPS solves on the mesh moved by the smooth map
+   x -> x + EPS sin(pi x) sin(pi y) sin(pi z) (1, 1, 1) (3-D; it fixes the boundary, so the domain stays the unit cube) */
 static int g_coefficient = 0, g_profile = 0, g_dim = 3;
-static double g_tol = 1e-12;
+static double g_tol = 1e-12, g_distort = 0.0;
 static void common_options(int argc, char **argv)
 {
   g_coefficient = arg_int(argc, argv, "--coefficient", 0);
   g_profile = arg_int(argc, argv, "--profile", 0);
   g_tol = arg_double(argc, argv, "--tol", 1e-12);
+  g_distort = arg_double(argc, argv, "--distort", 0.0);
+}
+
+/* the level's operator: on the unit cube, or with --distort on the smoothly mapped mesh of n^3 cells (its vertices are the
+   map of the uniform grid, so the meshes of the h-levels are nested) */
+static int create_level_operator(pmg_context *ctx, const level_t *lv, pmg_operator **op)
+{
+  if (g_distort == 0.0)
+    return pmg_laplace_operator_create(ctx, g_dim, lv->degree, lv->n, lv->n, lv->n, PMG_ALL_FACES, g_coefficient, op);
+  if (g_dim != 3) {
+    fprintf(stderr, "--distort: the mapped operator is 3-D only\n");
+    return PMG_ERR_UNSUPPORTED;
+  }
+  const int n = lv->n, nv = n + 1;
+  double *v = (double *)malloc(sizeof(double) * 3 * nv * nv * nv);
+  if (!v) return PMG_ERR_NOMEM;
+  const double pi = 3.14159265358979323846;
+  for (int k = 0; k < nv; ++k)
+    for (int j = 0; j < nv; ++j)
+      for (int i = 0; i < nv; ++i) {
+        const double x = (double)i / n, y = (double)j / n, z = (double)k / n;
+        const double s = g_distort * sin(pi * x) * sin(pi * y) * sin(pi * z);
+        double *p = v + 3 * ((size_t)i + (size_t)nv * (j + (size_t)nv * k));
+        p[0] = x + s; p[1] = y + s; p[2] = z + s;
+      }
+  const int rc = pmg_laplace_operator_create_mapped(ctx, lv->degree, n, n, n, PMG_ALL_FACES, g_coefficient, v, op);
+  free(v);
+  return rc;
 }
 
 static long long n_dofs_of(int degree, int n)
@@ -116,8 +145,8 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
   pmg_transfer *tr[MAXL];
   pmg_chebyshev *sm[MAXL];
   memset(tr, 0, sizeof(tr));
-  for (int l = 0; l < L; ++l)
-    CK(pmg_laplace_operator_create(ctx, g_dim, lv[l].degree, lv[l].n, lv[l].n, lv[l].n, PMG_ALL_FACES, g_coefficient, &ops[l]));
+  if (g_distort != 0.0) RPRINT("  mapped mesh: x + %g sin(pi x) sin(pi y) sin(pi z) (1, 1, 1)\n", g_distort);
+  for (int l = 0; l < L; ++l) CK(create_level_operator(ctx, &lv[l], &ops[l]));
   for (int l = 1; l < L; ++l) {
     if (lv[l].degree == lv[l - 1].degree) CK(pmg_transfer_create_geometric(ops[l - 1], ops[l], &tr[l]));
     else CK(pmg_transfer_create_polynomial(ops[l - 1], ops[l], &tr[l]));

@@ -150,7 +150,10 @@ struct pmg_operator {
   pmg_layout lay;
   pmgk_level lv;
   double *d_dinv_tab;
-  double *d_coef;        /* variable coefficient at the quadrature points (coefficient != 0) */
+  double *d_coef;        /* variable coefficient at the quadrature points (coefficient != 0), or the six grids of the
+                            mapped geometry's G_q (mapped) */
+  int mapped;            /* created by pmg_laplace_operator_create_mapped: lv.geo_stride != 0 where the level is stored */
+  double *d_vert;        /* mapped: vertex planes lv.coef_cz0 .. lv.cz_hi of the stored cell layers (rhs, solution norm) */
   pmg_vector *dinv;      /* explicit inverse diagonal once compute_diagonal() ran */
   pmg_vector *cg_ws[4];  /* CG work vectors r, z, p, Ap: created by the first pmg_cg_solve, kept until destroy */
 };

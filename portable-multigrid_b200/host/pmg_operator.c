@@ -44,8 +44,63 @@ static int setup_coefficient(pmg_operator *op)
   return PMG_OK;
 }
 
-int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz,
-                                unsigned faces, int coefficient, pmg_operator **out)
+/* Mapped geometry (SURVEY.md row f4): the six entries of G_q = w_q a(x_q) |det J_q| J_q^-1 J_q^-T of every quadrature point
+   of the locally stored cell layers, computed on the device from the trilinear maps of the cells (csrc/pmg_apply_geo.cu)
+   and streamed by the tensor variant of the variable-coefficient kernel.  Only the vertex planes of the stored layers are
+   uploaded; a cell with det J <= 0 at a Gauss point or a non-finite vertex rejects the mesh. */
+static int geo_diagonal(pmg_operator *op)
+{
+  const int n1 = op->degree + 1;
+  double Sq[PMGK_MAX_N1 * PMGK_MAX_N1], G[PMGK_MAX_N1 * PMGK_MAX_N1], SG[PMGK_MAX_N1 * PMGK_MAX_N1];
+  pmg_fe_shape_tables(op->degree, Sq, NULL, G, NULL, NULL);
+  for (int i = 0; i < n1 * n1; ++i) { SG[i] = Sq[i] * G[i]; Sq[i] *= Sq[i]; G[i] *= G[i]; }
+  return pmgk_geo_fill_dinv(&op->lv, Sq, G, SG, op->dinv->d, op->ctx->stream);
+}
+
+static int setup_geometry(pmg_operator *op, const double *vertices)
+{
+  pmgk_level *lv = &op->lv;
+  double gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
+  pmg_fe_shape_tables(op->degree, lv->Sq, lv->Dco, NULL, gq, gw);
+  lv->coef_cz0 = lv->z0 / op->degree;
+  PMG_CHECK(pmg_vector_create_layout(op->ctx, &op->lay, &op->dinv));
+  if (!op->lay.active) return PMG_OK;
+  const int64_t n = pmgk_var_coef_doubles(lv);
+  lv->geo_stride = n;
+  if (cudaMalloc((void **)&op->d_coef, sizeof(double) * 6 * (size_t)n) != cudaSuccess) {
+    pmg_set_error("cudaMalloc of %lld geometry values failed", (long long)(6 * n));
+    return PMG_ERR_NOMEM;
+  }
+  lv->coef = op->d_coef;
+  /* vertex planes coef_cz0 .. cz_hi of the stored cell layers, and one error word */
+  const size_t vplane = (size_t)(lv->nx + 1) * (lv->ny + 1) * 3;
+  const size_t nv = vplane * (size_t)(lv->cz_hi - lv->coef_cz0 + 1);
+  cudaStream_t st = op->ctx->stream;
+  unsigned long long *d_err = NULL, h_err = 0;
+  int rc = PMG_OK;
+  if (cudaMalloc((void **)&op->d_vert, sizeof(double) * nv + sizeof(unsigned long long)) != cudaSuccess) {
+    pmg_set_error("cudaMalloc of %lld vertex coordinates failed", (long long)nv);
+    return PMG_ERR_NOMEM;
+  }
+  d_err = (unsigned long long *)(op->d_vert + nv);
+  if (cudaMemcpyAsync(op->d_vert, vertices + vplane * lv->coef_cz0, sizeof(double) * nv, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+      cudaMemsetAsync(d_err, 0xFF, sizeof(unsigned long long), st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (rc == PMG_OK) rc = pmgk_geo_fill(lv, op->coefficient, op->d_vert, gq, gw, op->d_coef, d_err, st);
+  if (rc == PMG_OK && cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* vertices and h_err are pageable */
+  if (rc != PMG_OK) return rc;
+  if (h_err != ~0ull) {
+    const long long c = (long long)h_err, cx = c % lv->nx, cy = c / lv->nx % lv->ny, cz = c / ((long long)lv->nx * lv->ny);
+    pmg_set_error("mapped mesh: cell %lld = (%lld, %lld, %lld) has det J <= 0 at a Gauss point or a non-finite vertex", c, cx, cy, cz);
+    return PMG_ERR_ARG;
+  }
+  PMG_CHECK(geo_diagonal(op));
+  lv->dinv_vec = op->dinv->d;
+  return PMG_OK;
+}
+
+static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz, unsigned faces, int coefficient,
+                           const double *vertices, pmg_operator **out)
 {
   if (!ctx || !out || nx < 1 || ny < 1 || nz < 1) { pmg_set_error("operator_create: bad arguments"); return PMG_ERR_ARG; }
   if (dim != 2 && dim != 3) { pmg_set_error("dim = %d: the reference instantiates dim = 2 and dim = 3", dim); return PMG_ERR_UNSUPPORTED; }
@@ -57,6 +112,7 @@ int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, i
   pmg_operator *op = (pmg_operator *)calloc(1, sizeof(*op));
   if (!op) return PMG_ERR_NOMEM;
   op->ctx = ctx; op->dim = dim; op->degree = degree; op->coefficient = coefficient; op->faces = faces & PMG_ALL_FACES;
+  op->mapped = vertices != NULL;
   PMG_CHECK(pmg_layout_make(ctx, dim, degree, nx, ny, nz, &op->lay));
   pmgk_level *lv = &op->lv;
   lv->dim = dim;
@@ -83,12 +139,28 @@ int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, i
   lv->dinv_vec = NULL;
   const char *tv = getenv("PMG_TILE_VARIANT");
   lv->tile_variant = tv ? atoi(tv) : 0;
-  if (coefficient != 0) {
+  if (vertices) {
+    const int rc = setup_geometry(op, vertices);
+    if (rc != PMG_OK) { pmg_laplace_operator_destroy(op); return rc; }
+  } else if (coefficient != 0) {
     const int rc = setup_coefficient(op);
     if (rc != PMG_OK) { pmg_laplace_operator_destroy(op); return rc; }
   }
   *out = op;
   return PMG_OK;
+}
+
+int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz,
+                                unsigned faces, int coefficient, pmg_operator **out)
+{
+  return operator_create(ctx, dim, degree, nx, ny, nz, faces, coefficient, NULL, out);
+}
+
+int pmg_laplace_operator_create_mapped(pmg_context *ctx, int degree, int nx, int ny, int nz, unsigned faces, int coefficient,
+                                       const double *vertices, pmg_operator **out)
+{
+  if (!vertices) { pmg_set_error("operator_create_mapped: no vertices"); return PMG_ERR_ARG; }
+  return operator_create(ctx, 3, degree, nx, ny, nz, faces, coefficient, vertices, out);
 }
 
 int pmg_laplace_operator_destroy(pmg_operator *op)
@@ -99,6 +171,7 @@ int pmg_laplace_operator_destroy(pmg_operator *op)
   for (int i = 0; i < 4; ++i) if (op->cg_ws[i]) pmg_vector_destroy(op->cg_ws[i]);
   cudaFree(op->d_dinv_tab);
   cudaFree(op->d_coef);
+  cudaFree(op->d_vert);
   free(op);
   return PMG_OK;
 }
@@ -247,6 +320,7 @@ int pmg_laplace_operator_compute_diagonal(pmg_operator *op)
   if (!op) return PMG_ERR_ARG;
   if (!op->dinv) PMG_CHECK(pmg_vector_create_layout(op->ctx, &op->lay, &op->dinv));
   if (!op->lay.active) return PMG_OK;
+  if (op->lv.geo_stride) return geo_diagonal(op);
   if (op->coefficient != 0) return var_diagonal(op);
   /* diagonal of the tensor-product cell matrices summed at shared dofs, 1 on constrained dofs,
      inverted (:752-917).  The fused smoother keeps using the (p+2)^3 table: same numbers,
@@ -312,6 +386,54 @@ int pmg_laplace_operator_vmult_host(const pmg_operator *op, double *dst_host, co
 }
 
 /* ---- driver helpers: right-hand side and solution norm ---------------------------------- */
+/* Mapped mesh: neither the load vector nor the norm factorises.  b_i = sum_cells sum_q phi_i(x_q) w_q |det J_q| (QGauss(p+1),
+   constrained rows dropped) as a deterministic per-dof gather over the <= 8 cells of each dof; the ghost planes are then
+   refreshed from their owners. */
+static int mapped_rhs(const pmg_operator *op, pmg_vector *rhs)
+{
+  const pmgk_level *lv = &op->lv;
+  if (!op->lay.active) return PMG_OK;
+  double S[PMGK_MAX_N1 * PMGK_MAX_N1], gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
+  pmg_fe_shape_tables(op->degree, S, NULL, NULL, gq, gw);
+  cudaStream_t st = op->ctx->stream;
+  double *W = NULL;
+  const int64_t n = pmgk_var_coef_doubles(lv);
+  if (cudaMallocAsync((void **)&W, sizeof(double) * (size_t)(n > 0 ? n : 1), st) != cudaSuccess) return PMG_ERR_NOMEM;
+  int rc = pmgk_geo_rhs(lv, op->d_vert, S, gq, gw, W, rhs->d, st);
+  cudaFreeAsync(W, st);
+  if (rc != PMG_OK) return rc;
+  return pmg_halo_update(op->ctx, &op->lay, rhs->d);
+}
+
+/* ||u_h||_L2 with QGauss(p+2) as integrate_difference (program.cc:382-395): per owned cell u_h interpolated to the (p+2)^3
+   points, weighted with w |det J|; the cell sums are reduced deterministically (two-stage) and over the ranks */
+static int mapped_norm(const pmg_operator *op, const pmg_vector *u, double *norm)
+{
+  pmg_context *ctx = op->ctx;
+  const pmgk_level *lv = &op->lv;
+  const int p = op->degree, n1 = p + 1, m = p + 2;
+  double gll[PMG_MAX_DEGREE + 2], g[PMG_MAX_DEGREE + 2], w[PMG_MAX_DEGREE + 2], E[(PMG_MAX_DEGREE + 2) * (PMG_MAX_DEGREE + 1)];
+  pmg_fe_gll(n1, gll);
+  pmg_fe_gauss(m, g, w);
+  for (int q = 0; q < m; ++q) pmg_fe_lagrange(n1, gll, g[q], E + q * n1, NULL);
+  PMG_CUDA(cudaMemsetAsync(ctx->scalars, 0, sizeof(double), ctx->stream));
+  if (op->lay.active) {
+    const int64_t ncells = (int64_t)lv->nx * lv->ny * (lv->cz_hi - lv->cz_lo);
+    double *sums = NULL;
+    PMG_CHECK(pmg_halo_update(ctx, &u->lay, u->d));
+    if (cudaMallocAsync((void **)&sums, sizeof(double) * (size_t)(ncells > 0 ? ncells : 1), ctx->stream) != cudaSuccess) return PMG_ERR_NOMEM;
+    int rc = pmgk_geo_norm_cells(lv, op->d_vert, E, g, w, u->d, sums, ctx->stream);
+    if (rc == PMG_OK) rc = pmgk_sum(sums, ncells, ctx->scalars, ctx->work, ctx->stream);
+    cudaFreeAsync(sums, ctx->stream);
+    if (rc != PMG_OK) return rc;
+  }
+  PMG_CHECK(pmg_allreduce_sum(ctx, ctx->scalars, 1));
+  PMG_CUDA(cudaMemcpyAsync(ctx->h_scalars, ctx->scalars, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  PMG_CUDA(cudaStreamSynchronize(ctx->stream));
+  *norm = sqrt(fabs(ctx->h_scalars[0]));
+  return PMG_OK;
+}
+
 /* Load vector of f = 1 (reference source/geometric_multigrid/program.cc:289-334).  On the box mesh
    the cell vector is the tensor product of the 1-D load b1[i] = sum_q w_q phi_i(x_q) h, so the global
    vector is separable too: rhs(x,y,z) = bx(x) by(y) bz(z), constrained rows dropped.  Assembled on
@@ -320,6 +442,7 @@ int pmg_laplace_operator_assemble_rhs(const pmg_operator *op, pmg_vector *rhs)
 {
   if (!op) return PMG_ERR_ARG;
   PMG_CHECK(check_vec(op, rhs, "assemble_rhs"));
+  if (op->mapped) return mapped_rhs(op, rhs);
   const pmg_layout *l = &op->lay;
   if (!l->active) return PMG_OK;
   const int p = op->degree, n1 = p + 1;
@@ -369,6 +492,7 @@ int pmg_laplace_operator_solution_norm(const pmg_operator *op, const pmg_vector 
 {
   if (!op || !norm) return PMG_ERR_ARG;
   PMG_CHECK(check_vec(op, u, "solution_norm"));
+  if (op->mapped) return mapped_norm(op, u, norm);
   pmg_context *ctx = op->ctx;
   pmg_vector *t = NULL;
   PMG_CHECK(pmg_vector_create_layout(ctx, &op->lay, &t));

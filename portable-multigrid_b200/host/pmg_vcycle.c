@@ -152,7 +152,7 @@ static void choose_coarse_top(pmg_vcycle *v)
     const pmg_operator *op = v->op[l];
     if (!pmgk_coarse_cycle_supported(&op->lv) && op->lay.active) break;
     if (op->ctx->n_ranks > 1 && !op->lay.gathered) break;
-    if (op->degree != v->op[0]->degree || op->coefficient != 0 || op->dim != 3) break;
+    if (op->degree != v->op[0]->degree || op->coefficient != 0 || op->mapped || op->dim != 3) break;
     if (l > 0 && v->tr[l]->kind != 0) break;
     const double n1 = op->degree + 1;
     const char *w = getenv("PMG_COARSE_MAX_WORK");

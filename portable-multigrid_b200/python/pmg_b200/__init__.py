@@ -219,14 +219,28 @@ class Vector:
 class LaplaceOperator:
     """Portable::LaplaceOperator (reference include/operators/portable_laplace_operator.h:383-461)."""
 
-    def __init__(self, ctx, degree, n, dirichlet_faces=PMG_ALL_FACES, dim=3, coefficient=0):
+    def __init__(self, ctx, degree, n, dirichlet_faces=PMG_ALL_FACES, dim=3, coefficient=0, vertices=None):
+        """vertices: None (the unit cube cut into equal boxes) or the (nx+1)(ny+1)(nz+1) mesh vertices of a deformed
+        structured mesh, shape (nz+1, ny+1, nx+1, 3) or flat in that order (pmg_laplace_operator_create_mapped); 3-D only."""
         if isinstance(n, int):
             n = (n,) * dim
         n = tuple(n) + (1,) * (3 - len(n))  # dim = 2: (nx, ny); the C-ABI ignores nz
         self.ctx, self.degree, self.ncells, self.dim = ctx, degree, tuple(n), dim
         self.h = _vp()
-        _ck(lib().pmg_laplace_operator_create(ctx.h, C.c_int(dim), C.c_int(degree), C.c_int(n[0]), C.c_int(n[1]),
-                                              C.c_int(n[2]), C.c_uint(dirichlet_faces), C.c_int(coefficient), C.byref(self.h)))
+        self.vertices = None
+        if vertices is None:
+            _ck(lib().pmg_laplace_operator_create(ctx.h, C.c_int(dim), C.c_int(degree), C.c_int(n[0]), C.c_int(n[1]),
+                                                  C.c_int(n[2]), C.c_uint(dirichlet_faces), C.c_int(coefficient), C.byref(self.h)))
+            return
+        if dim != 3:
+            raise PmgError(-3, "the mapped operator is 3-D only (dim = %d)" % dim)
+        v = np.ascontiguousarray(vertices, dtype=np.float64).reshape(-1)
+        if v.size != 3 * (n[0] + 1) * (n[1] + 1) * (n[2] + 1):
+            raise PmgError(-1, "vertices: %d values for %d x %d x %d cells, need 3 (nx+1)(ny+1)(nz+1)" % (v.size, *n))
+        self.vertices = v.reshape(n[2] + 1, n[1] + 1, n[0] + 1, 3)
+        _ck(lib().pmg_laplace_operator_create_mapped(ctx.h, C.c_int(degree), C.c_int(n[0]), C.c_int(n[1]), C.c_int(n[2]),
+                                                     C.c_uint(dirichlet_faces), C.c_int(coefficient), _np_ptr(v),
+                                                     C.byref(self.h)))
 
     def __del__(self):
         try:
@@ -406,12 +420,15 @@ def cg_solve(A, x, b, precond=None, max_iterations=None, tolerance=None, rel_tol
 
 
 def build_hierarchy(ctx, levels, pre=2, post=2, degree=5, smoothing_range=15.0, eig_cg_n_iterations=10,
-                    coarse_range=1e-3, faces=PMG_ALL_FACES, coefficient=0, dim=3):
+                    coarse_range=1e-3, faces=PMG_ALL_FACES, coefficient=0, dim=3, vertices=None):
     """levels: list of (degree, n_cells) coarse -> fine; consecutive levels must be related by one
     global refinement (h) or a degree change on the same mesh (p).  Smoother parameters as in the
     reference drivers (program.cc:267-279).  coefficient = 1: every level discretises -div(a grad u) with
-    a = 1/(0.05 + 2|x|^2) at its own quadrature points (BASELINE config 5)."""
-    ops = [LaplaceOperator(ctx, p, n, faces, dim=dim, coefficient=coefficient) for (p, n) in levels]
+    a = 1/(0.05 + 2|x|^2) at its own quadrature points (BASELINE config 5).  vertices: the finest mesh's vertices
+    (LaplaceOperator); a coarser mesh takes every 2^k-th vertex in each direction (nested meshes), p-levels share them."""
+    ops = [LaplaceOperator(ctx, p, n, faces, dim=dim, coefficient=coefficient,
+                           vertices=None if vertices is None else mesh_vertices_coarsened(vertices, levels[-1][1], n))
+           for (p, n) in levels]
     transfers = []
     for l in range(1, len(levels)):
         if levels[l][0] == levels[l - 1][0]:
@@ -430,6 +447,27 @@ def build_hierarchy(ctx, levels, pre=2, post=2, degree=5, smoothing_range=15.0, 
 
 
 # ---- host-only helpers (no GPU needed) -------------------------------------------------------
+def mesh_vertices_coarsened(vertices, n_fine, n_coarse):
+    """The vertices of the coarse mesh of a nested pair: vertex (i, j, k) of the coarse mesh is vertex (f i, f j, f k)
+    of the fine one, f = n_fine / n_coarse per direction (a power of two)."""
+    nf = (n_fine,) * 3 if isinstance(n_fine, int) else tuple(n_fine)
+    nc = (n_coarse,) * 3 if isinstance(n_coarse, int) else tuple(n_coarse)
+    v = np.asarray(vertices, dtype=np.float64).reshape(nf[2] + 1, nf[1] + 1, nf[0] + 1, 3)
+    f = []
+    for a, b in zip(nf, nc):
+        if b < 1 or a % b or (a // b) & (a // b - 1):
+            raise PmgError(-1, "mesh of %s cells is not a refinement of %s cells" % (nf, nc))
+        f.append(a // b)
+    return np.ascontiguousarray(v[:: f[2], :: f[1], :: f[0]])
+
+
+def mesh_vertices_uniform(n, box=(1.0, 1.0, 1.0)):
+    """Vertices of the box [0, box] cut into n equal cells per direction, shape (nz+1, ny+1, nx+1, 3)."""
+    n = (n,) * 3 if isinstance(n, int) else tuple(n)
+    z, y, x = np.meshgrid(*[np.arange(n[d] + 1) * (box[d] / n[d]) for d in (2, 1, 0)], indexing="ij")
+    return np.ascontiguousarray(np.stack([x, y, z], axis=-1))
+
+
 def host_fastdiag_tables(p):
     n = p + 1
     S, lam = np.zeros(n * n), np.zeros(n)
