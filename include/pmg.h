@@ -96,6 +96,20 @@ int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, i
    (inverted or degenerate) or a vertex that is not finite; PMG_ERR_UNSUPPORTED for degrees outside 1..PMG_MAX_DEGREE. */
 int pmg_laplace_operator_create_mapped(pmg_context *ctx, int degree, int nx, int ny, int nz, unsigned dirichlet_faces,
                                        int coefficient, const double *vertices, pmg_operator **op);
+/* The Laplace operator (coefficient 0 or 1 as above) on a structured mesh of nx x ny x nz curved hexahedra, 3-D only: the
+   geometry MappingQ(k) gives the cells of a mesh on a curved manifold (a cylinder, a shell, a pipe bend).  nodes: HOST array
+   of the (nx k + 1)(ny k + 1)(nz k + 1) geometry support points, (x, y, z) interleaved, in global lexicographic order
+   (x fastest), the same full array on every rank; it is read during the call only.  Cell (cx, cy, cz) is the
+   tensor-product Lagrange interpolant of degree k = geometry_degree through the nodes (cx k + i, cy k + j, cz k + l),
+   0 <= i, j, l <= k, placed at the Gauss-Lobatto points of FE_Q(k) (pmg_host_support_points).  k = degree: the nodes are
+   the DoF support points, the MappingQ(degree) the reference's operator builds; k = 1: the array is the vertex array of
+   pmg_laplace_operator_create_mapped, with the same result.  Everything else as pmg_laplace_operator_create_mapped; the
+   h-transfer and p-transfer are reference-cell contractions, so the meshes of an h-hierarchy need not be nested: each
+   level interpolates the manifold itself, as MappingQ on every level does.
+   Errors: PMG_ERR_ARG with the first offending cell in pmg_last_error() if a cell has det J <= 0 at one of its Gauss points
+   or a node that is not finite; PMG_ERR_UNSUPPORTED for degree or geometry_degree outside 1..PMG_MAX_DEGREE. */
+int pmg_laplace_operator_create_curved(pmg_context *ctx, int degree, int geometry_degree, int nx, int ny, int nz,
+                                       unsigned dirichlet_faces, int coefficient, const double *nodes, pmg_operator **op);
 int pmg_laplace_operator_destroy(pmg_operator *op);
 int pmg_laplace_operator_vmult(const pmg_operator *op, pmg_vector *dst, const pmg_vector *src);  /* :557-719 */
 int pmg_laplace_operator_Tvmult(const pmg_operator *op, pmg_vector *dst, const pmg_vector *src); /* :721-735 */
@@ -193,6 +207,9 @@ int pmg_cg_solve(const pmg_operator *A, pmg_vector *x, const pmg_vector *b, pmg_
 /* 1-D tables for FE_Q(degree): S (n1*n1, M = S^T S, K = S^T diag(lam) S), lam (n1) */
 int pmg_host_fastdiag_tables(int degree, double *S, double *lam);
 int pmg_host_pencil(int degree, double *M, double *K);
+/* the degree + 1 Gauss-Lobatto points of [0, 1] (support points of FE_Q(degree)): where the nodes of a curved cell sit on the
+   reference cell, i.e. where a caller evaluates its manifold for pmg_laplace_operator_create_curved */
+int pmg_host_support_points(int degree, double *x);
 int pmg_host_prolongation_1d(int kind, int degree_coarse, int degree_fine, double *P);
 /* z-slab decomposition: owned cell layers of `rank` on a level with nz layers */
 int pmg_host_partition(int nz, int n_ranks, int rank, int *cz_lo, int *cz_hi);

@@ -42,7 +42,7 @@ typedef struct pmgk_level {
   double Sq[PMGK_MAX_N1 * PMGK_MAX_N1];  /* shape values phi_i(x_q), row q (Gauss point), column i (n1 x n1) */
   double Dco[PMGK_MAX_N1 * PMGK_MAX_N1]; /* co_shape_gradients: derivative of Gauss-point Lagrange basis r at Gauss point q */
   /* mapped geometry (0 = the box's affine cells): coef then holds six grids of the layout above, geo_stride doubles apart --
-     the entries xx, xy, xz, yy, yz, zz of  G_q = w_q a(x_q) |det J_q| J_q^-1 J_q^-T  of the cells' trilinear maps */
+     the entries xx, xy, xz, yy, yz, zz of  G_q = w_q a(x_q) |det J_q| J_q^-1 J_q^-T  of the cells' trilinear or curved maps */
   int64_t geo_stride;
 } pmgk_level;
 
@@ -87,24 +87,27 @@ int pmgk_var_fill_coef(const pmgk_level *lv, int kind, const double *gq, const d
    S2 / G2: HOST n1 x n1 tables, squared shape values / squared nodal shape gradients at the Gauss points, row q */
 int pmgk_var_fill_dinv(const pmgk_level *lv, const double *S2, const double *G2, double *dinv, void *stream);
 
-/* mapped-geometry set-up (csrc/pmg_apply_geo.cu).  vert: device, the vertex planes coef_cz0 .. cz_hi of the level,
-   (nx+1) x (ny+1) points per plane, x fastest, (x, y, z) interleaved; kind 0: a = 1, 1: the C5 coefficient at the mapped
-   point; gq / gw: HOST Gauss points / weights on [0,1]; geo: device, 6 pmgk_var_coef_doubles(lv) doubles (lv->geo_stride
-   must be pmgk_var_coef_doubles(lv)).  err: device word, ~0 on entry; on return (when the stream has run) it holds the
-   smallest global index cx + nx (cy + ny cz) of a cell with det J <= 0 at a Gauss point or a non-finite vertex, else ~0. */
-int pmgk_geo_fill(const pmgk_level *lv, int kind, const double *vert, const double *gq, const double *gw, double *geo,
+/* mapped-geometry set-up (csrc/pmg_apply_geo.cu).  k: the geometry degree, 1 = trilinear cells, 2 .. PMGK_MAX_N1-1 = curved
+   cells, each the Lagrange interpolant of degree k through (k+1)^3 nodes at the Gauss-Lobatto points (MappingQ(k)).  vert:
+   device, the node planes k coef_cz0 .. k cz_hi of the level, (nx k+1) x (ny k+1) points per plane, x fastest, (x, y, z)
+   interleaved (k = 1: the vertex planes); kind 0: a = 1, 1: the C5 coefficient at the mapped point; gq / gw: HOST Gauss
+   points / weights on [0,1]; geo: device, 6 pmgk_var_coef_doubles(lv) doubles (lv->geo_stride must be
+   pmgk_var_coef_doubles(lv)).  err: device word, ~0 on entry; on return (when the stream has run) it holds the smallest
+   global index cx + nx (cy + ny cz) of a cell with det J <= 0 at a Gauss point or a non-finite node, else ~0. */
+int pmgk_geo_fill(const pmgk_level *lv, int k, int kind, const double *vert, const double *gq, const double *gw, double *geo,
                   unsigned long long *err, void *stream);
 /* inverse diagonal of the mapped operator; S2 / G2 as pmgk_var_fill_dinv, SG: HOST table S(q,i) G(q,i) */
 int pmgk_geo_fill_dinv(const pmgk_level *lv, const double *S2, const double *G2, const double *SG, double *dinv, void *stream);
 
 /* load vector of f = 1 on the mapped mesh on all stored planes (constrained rows 0; a ghost plane holds the part of the
-   stored cells only): vert as pmgk_geo_fill; S: HOST n1 x n1 shape values [q][i], gq / gw: HOST Gauss points / weights;
+   stored cells only): k, vert as pmgk_geo_fill; S: HOST n1 x n1 shape values [q][i], gq / gw: HOST Gauss points / weights;
    W: device scratch of pmgk_var_coef_doubles(lv) doubles */
-int pmgk_geo_rhs(const pmgk_level *lv, const double *vert, const double *S, const double *gq, const double *gw, double *W,
+int pmgk_geo_rhs(const pmgk_level *lv, int k, const double *vert, const double *S, const double *gq, const double *gw, double *W,
                  double *rhs, void *stream);
 /* integral of u^2 over each owned cell of the mapped mesh with QGauss(p+2): cell_sums[c], c = cx + nx (cy + ny (cz - cz_lo));
-   E: HOST (p+2) x (p+1) values phi_i(x_q), gq / gw: HOST the p+2 Gauss points / weights; u: local vector, ghosts current */
-int pmgk_geo_norm_cells(const pmgk_level *lv, const double *vert, const double *E, const double *gq, const double *gw,
+   k, vert as pmgk_geo_fill; E: HOST (p+2) x (p+1) values phi_i(x_q), gq / gw: HOST the p+2 Gauss points / weights; u: local
+   vector, ghosts current */
+int pmgk_geo_norm_cells(const pmgk_level *lv, int k, const double *vert, const double *E, const double *gq, const double *gw,
                         const double *u, double *cell_sums, void *stream);
 
 /* inverse diagonal as an explicit vector (LaplaceOperator::compute_diagonal, :752-917) */

@@ -25,6 +25,7 @@
 //
 // Written against the same executor as the other tile programs: runs under tests/emu on the CPU test-suite.
 #pragma once
+#include <math.h>
 #include <type_traits>
 #include "pmg_apply_tile.h"
 
@@ -134,20 +135,12 @@ PMG_HD double pmg_geo_diag_entry(int gx, int gy, int gz, int nx, int ny, int cz_
   return diag;
 }
 
-// G_q of one quadrature point of the trilinear map of a cell: v[c][d] = coordinate d of the cell's vertex
-// c = ix + 2 iy + 4 iz; (xq, yq, zq) = the point on the reference cell [0,1]^3; wq = quadrature weight.  Writes the
-// six entries (xx, xy, xz, yy, yz, zz) of  wq a(x) |det J| J^-1 J^-T  (a = C5 coefficient at the mapped point when
-// c5 != 0, else 1) and returns det J (<= 0 or NaN: the cell is inverted or degenerate)
-PMG_HD double pmg_geo_point(const double (*v)[3], double xq, double yq, double zq, double wq, int c5, double *G)
+// G_q of one quadrature point from the map's Jacobian J (J[d][e] = d x_d / d xi_e) and the mapped point x; wq = quadrature
+// weight.  Writes the six entries (xx, xy, xz, yy, yz, zz) of  wq a(x) |det J| J^-1 J^-T  (a = C5 coefficient at x when
+// c5 != 0, else 1) and returns det J (<= 0 or NaN: the cell is inverted or degenerate).  The one copy of this arithmetic:
+// the trilinear (pmg_geo_point) and the curved (pmg_curved_point) set-up both end here.
+PMG_HD double pmg_geo_tensor(const double (*J)[3], const double *x, double wq, int c5, double *G)
 {
-  const double L[2][3] = {{1.0 - xq, 1.0 - yq, 1.0 - zq}, {xq, yq, zq}};
-  double J[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}}, x[3] = {0, 0, 0}; // J[d][e] = d x_d / d xi_e
-  for (int c = 0; c < 8; ++c) {
-    const int i = c & 1, j = c >> 1 & 1, k = c >> 2;
-    const double w = L[i][0] * L[j][1] * L[k][2];
-    const double d0 = (i ? 1.0 : -1.0) * L[j][1] * L[k][2], d1 = L[i][0] * (j ? 1.0 : -1.0) * L[k][2], d2 = L[i][0] * L[j][1] * (k ? 1.0 : -1.0);
-    for (int d = 0; d < 3; ++d) { x[d] += w * v[c][d]; J[d][0] += d0 * v[c][d]; J[d][1] += d1 * v[c][d]; J[d][2] += d2 * v[c][d]; }
-  }
   // adjugate: J^-1 = adj(J) / det
   const double A00 = J[1][1] * J[2][2] - J[1][2] * J[2][1], A01 = J[0][2] * J[2][1] - J[0][1] * J[2][2], A02 = J[0][1] * J[1][2] - J[0][2] * J[1][1];
   const double A10 = J[1][2] * J[2][0] - J[1][0] * J[2][2], A11 = J[0][0] * J[2][2] - J[0][2] * J[2][0], A12 = J[0][2] * J[1][0] - J[0][0] * J[1][2];
@@ -162,6 +155,55 @@ PMG_HD double pmg_geo_point(const double (*v)[3], double xq, double yq, double z
   G[4] = f * (A10 * A20 + A11 * A21 + A12 * A22);
   G[5] = f * (A20 * A20 + A21 * A21 + A22 * A22);
   return det;
+}
+
+// G_q of one quadrature point of the trilinear map of a cell (pmg_geo_tensor): v[c][d] = coordinate d of the cell's
+// vertex c = ix + 2 iy + 4 iz; (xq, yq, zq) = the point on the reference cell [0,1]^3; wq = quadrature weight
+PMG_HD double pmg_geo_point(const double (*v)[3], double xq, double yq, double zq, double wq, int c5, double *G)
+{
+  const double L[2][3] = {{1.0 - xq, 1.0 - yq, 1.0 - zq}, {xq, yq, zq}};
+  double J[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}}, x[3] = {0, 0, 0}; // J[d][e] = d x_d / d xi_e
+  for (int c = 0; c < 8; ++c) {
+    const int i = c & 1, j = c >> 1 & 1, k = c >> 2;
+    const double w = L[i][0] * L[j][1] * L[k][2];
+    const double d0 = (i ? 1.0 : -1.0) * L[j][1] * L[k][2], d1 = L[i][0] * (j ? 1.0 : -1.0) * L[k][2], d2 = L[i][0] * L[j][1] * (k ? 1.0 : -1.0);
+    for (int d = 0; d < 3; ++d) { x[d] += w * v[c][d]; J[d][0] += d0 * v[c][d]; J[d][1] += d1 * v[c][d]; J[d][2] += d2 * v[c][d]; }
+  }
+  return pmg_geo_tensor(J, x, wq, c5, G);
+}
+
+// x(xi) and J(xi) (J[d][e] = d x_d / d xi_e) of a curved cell at one reference point: the tensor-product Lagrange
+// interpolant of degree k through the cell's (k+1)^3 nodes at the Gauss-Lobatto points of FE_Q(k) (MappingQ(k)), by sum
+// factorisation -- contract x (values and derivatives), then y, then z.  Node (i, j, l) of the cell is at
+// node + 3 (i + j sy + l sz), (x, y, z) interleaved; Lx[i] / dLx[i] = value / derivative of the 1-D basis function i at the
+// point's xi_x, likewise for y and z.
+PMG_HD void pmg_curved_map(const double *node, int64_t sy, int64_t sz, int k, const double *Lx, const double *dLx,
+                           const double *Ly, const double *dLy, const double *Lz, const double *dLz, double *x, double (*J)[3])
+{
+  for (int d = 0; d < 3; ++d) { x[d] = 0.0; J[d][0] = 0.0; J[d][1] = 0.0; J[d][2] = 0.0; }
+  for (int l = 0; l <= k; ++l) {
+    double v[3] = {0, 0, 0}, vx[3] = {0, 0, 0}, vy[3] = {0, 0, 0}; // plane l contracted over x and y: value, d/dxi_x, d/dxi_y
+    for (int j = 0; j <= k; ++j) {
+      const double *row = node + 3 * (j * sy + l * sz);
+      double s[3] = {0, 0, 0}, sx[3] = {0, 0, 0};
+      for (int i = 0; i <= k; ++i)
+        for (int d = 0; d < 3; ++d) { s[d] += Lx[i] * row[3 * i + d]; sx[d] += dLx[i] * row[3 * i + d]; }
+      for (int d = 0; d < 3; ++d) { v[d] += Ly[j] * s[d]; vx[d] += Ly[j] * sx[d]; vy[d] += dLy[j] * s[d]; }
+    }
+    for (int d = 0; d < 3; ++d) { x[d] += Lz[l] * v[d]; J[d][0] += Lz[l] * vx[d]; J[d][1] += Lz[l] * vy[d]; J[d][2] += dLz[l] * v[d]; }
+  }
+}
+
+// G_q of one quadrature point of a curved cell (pmg_curved_map, then pmg_geo_tensor); the arguments as there.  Returns
+// det J, or -1 when a node of the cell is not finite (every node enters x(xi), so a non-finite node shows there).
+PMG_HD double pmg_curved_point(const double *node, int64_t sy, int64_t sz, int k, const double *Lx, const double *dLx,
+                               const double *Ly, const double *dLy, const double *Lz, const double *dLz, double wq, int c5,
+                               double *G)
+{
+  double x[3], J[3][3];
+  pmg_curved_map(node, sy, sz, k, Lx, dLx, Ly, dLy, Lz, dLz, x, J);
+  const double det = pmg_geo_tensor(J, x, wq, c5, G);
+  return isfinite(x[0] + x[1] + x[2]) && isfinite(det) ? det : -1.0;
 }
 
 // host side of the launchers (pmg_apply_var.cu, pmg_apply_geo.cu): number of z-chunks that minimises

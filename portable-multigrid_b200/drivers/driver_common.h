@@ -93,8 +93,12 @@ static double arg_double(int argc, char **argv, const char *name, double def)
 /* options shared by both drivers: --coefficient 1 solves -div(a grad u) = 1, a = 1/(0.05 + 2|x|^2) (BASELINE config 5),
    --tol T the relative CG tolerance (reference 1e-12, config 5: 1e-10), --profile 1 prints the per-level device time of one
    V-cycle (smoother / transfer / halo / other), --distort EPS solves on the mesh moved by the smooth map
-   x -> x + EPS sin(pi x) sin(pi y) sin(pi z) (1, 1, 1) (3-D; it fixes the boundary, so the domain stays the unit cube) */
-static int g_coefficient = 0, g_profile = 0, g_dim = 3;
+   x -> x + EPS sin(pi x) sin(pi y) sin(pi z) (1, 1, 1) (3-D; it fixes the boundary, so the domain stays the unit cube),
+   --shell 1 solves on the quarter cylindrical shell 1 <= r <= 2, 0 <= theta <= pi/2, 0 <= z <= 1 with Dirichlet conditions
+   on r = 1 and r = 2 and natural ones on the other faces (exact solution u = (1 - r^2)/4 + 3 ln r / (4 ln 2),
+   ||u||_L2 = 0.14143644722133), --mapping-degree K the geometry degree of the cells of --distort / --shell: 1 (default)
+   trilinear cells, 0 the level's FE degree (MappingQ(p) on every level), K >= 2 curved cells of degree K */
+static int g_coefficient = 0, g_profile = 0, g_dim = 3, g_shell = 0, g_mapping_degree = 1;
 static double g_tol = 1e-12, g_distort = 0.0;
 static void common_options(int argc, char **argv)
 {
@@ -102,32 +106,52 @@ static void common_options(int argc, char **argv)
   g_profile = arg_int(argc, argv, "--profile", 0);
   g_tol = arg_double(argc, argv, "--tol", 1e-12);
   g_distort = arg_double(argc, argv, "--distort", 0.0);
+  g_shell = arg_int(argc, argv, "--shell", 0);
+  g_mapping_degree = arg_int(argc, argv, "--mapping-degree", 1);
 }
 
-/* the level's operator: on the unit cube, or with --distort on the smoothly mapped mesh of n^3 cells (its vertices are the
-   map of the uniform grid, so the meshes of the h-levels are nested) */
+/* the level's operator: on the unit cube, or with --distort / --shell on the image of the unit cube's mesh of n^3 cells
+   under the map, with cells of geometry degree k: the map evaluated at the degree-k Gauss-Lobatto grid of every cell
+   (pmg_laplace_operator_create_curved; k = 1 gives the vertices of the trilinear cells, nested on the h-levels) */
 static int create_level_operator(pmg_context *ctx, const level_t *lv, pmg_operator **op)
 {
-  if (g_distort == 0.0)
+  if (g_distort == 0.0 && !g_shell)
     return pmg_laplace_operator_create(ctx, g_dim, lv->degree, lv->n, lv->n, lv->n, PMG_ALL_FACES, g_coefficient, op);
   if (g_dim != 3) {
-    fprintf(stderr, "--distort: the mapped operator is 3-D only\n");
+    fprintf(stderr, "--distort / --shell: the mapped operator is 3-D only\n");
     return PMG_ERR_UNSUPPORTED;
   }
-  const int n = lv->n, nv = n + 1;
-  double *v = (double *)malloc(sizeof(double) * 3 * nv * nv * nv);
-  if (!v) return PMG_ERR_NOMEM;
+  const int k = g_mapping_degree == 0 ? lv->degree : g_mapping_degree;
+  double s1[PMG_MAX_DEGREE + 1];
+  if (k < 1 || k > PMG_MAX_DEGREE) {
+    fprintf(stderr, "--mapping-degree %d outside 0..%d\n", g_mapping_degree, PMG_MAX_DEGREE);
+    return PMG_ERR_UNSUPPORTED;
+  }
+  pmg_host_support_points(k, s1);
+  const int n = lv->n, nv = n * k + 1;
+  double *v = (double *)malloc(sizeof(double) * 3 * nv * nv * nv), *t = (double *)malloc(sizeof(double) * nv);
+  if (!v || !t) { free(v); free(t); return PMG_ERR_NOMEM; }
+  for (int c = 0; c < n; ++c)
+    for (int i = 0; i < k; ++i) t[c * k + i] = (c + s1[i]) / n;
+  t[n * k] = 1.0;
   const double pi = 3.14159265358979323846;
-  for (int k = 0; k < nv; ++k)
+  for (int kz = 0; kz < nv; ++kz)
     for (int j = 0; j < nv; ++j)
       for (int i = 0; i < nv; ++i) {
-        const double x = (double)i / n, y = (double)j / n, z = (double)k / n;
-        const double s = g_distort * sin(pi * x) * sin(pi * y) * sin(pi * z);
-        double *p = v + 3 * ((size_t)i + (size_t)nv * (j + (size_t)nv * k));
-        p[0] = x + s; p[1] = y + s; p[2] = z + s;
+        const double x = t[i], y = t[j], z = t[kz];
+        double *p = v + 3 * ((size_t)i + (size_t)nv * (j + (size_t)nv * kz));
+        if (g_shell) {
+          const double r = 1.0 + x, th = 0.5 * pi * y;
+          p[0] = r * cos(th); p[1] = r * sin(th); p[2] = z;
+        } else {
+          const double s = g_distort * sin(pi * x) * sin(pi * y) * sin(pi * z);
+          p[0] = x + s; p[1] = y + s; p[2] = z + s;
+        }
       }
-  const int rc = pmg_laplace_operator_create_mapped(ctx, lv->degree, n, n, n, PMG_ALL_FACES, g_coefficient, v, op);
+  const unsigned faces = g_shell ? 0x3u : PMG_ALL_FACES;
+  const int rc = pmg_laplace_operator_create_curved(ctx, lv->degree, k, n, n, n, faces, g_coefficient, v, op);
   free(v);
+  free(t);
   return rc;
 }
 
@@ -145,7 +169,12 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
   pmg_transfer *tr[MAXL];
   pmg_chebyshev *sm[MAXL];
   memset(tr, 0, sizeof(tr));
-  if (g_distort != 0.0) RPRINT("  mapped mesh: x + %g sin(pi x) sin(pi y) sin(pi z) (1, 1, 1)\n", g_distort);
+  if (g_shell) RPRINT("  curved mesh: quarter cylindrical shell 1 <= r <= 2, 0 <= theta <= pi/2, 0 <= z <= 1\n");
+  else if (g_distort != 0.0) RPRINT("  mapped mesh: x + %g sin(pi x) sin(pi y) sin(pi z) (1, 1, 1)\n", g_distort);
+  if ((g_shell || g_distort != 0.0) && g_mapping_degree != 1) {
+    if (g_mapping_degree == 0) RPRINT("  geometry: MappingQ(p) cells, p the level's FE degree\n");
+    else RPRINT("  geometry: MappingQ(%d) cells\n", g_mapping_degree);
+  }
   for (int l = 0; l < L; ++l) CK(create_level_operator(ctx, &lv[l], &ops[l]));
   for (int l = 1; l < L; ++l) {
     if (lv[l].degree == lv[l - 1].degree) CK(pmg_transfer_create_geometric(ops[l - 1], ops[l], &tr[l]));

@@ -5,8 +5,8 @@
  * (:267-285, :342-343), CG to 1e-12 ||b|| (:345-352).  Prints the reference's lines (:189-199, :354-355, :395).
  * Flags: --degree D (only that degree), --max-degree M (default 7), --cycles C (default 6),
  *        --cheb-degree K (default 5; BASELINE config 1 uses 3), --pre/--post (default 2).
- *        --cells N (one run on N^dim cells, e.g. BASELINE config 4), --coefficient 1, --tol T, --profile 1, --distort EPS: see
- *        driver_common.h; --dim 2 runs the unit square (reference: dim = 3, :470).
+ *        --cells N (one run on N^dim cells, e.g. BASELINE config 4), --coefficient 1, --tol T, --profile 1, --distort EPS,
+ *        --shell 1, --mapping-degree K: see driver_common.h; --dim 2 runs the unit square (reference: dim = 3, :470).
  */
 #include "driver_common.h"
 

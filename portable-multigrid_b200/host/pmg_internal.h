@@ -152,8 +152,9 @@ struct pmg_operator {
   double *d_dinv_tab;
   double *d_coef;        /* variable coefficient at the quadrature points (coefficient != 0), or the six grids of the
                             mapped geometry's G_q (mapped) */
-  int mapped;            /* created by pmg_laplace_operator_create_mapped: lv.geo_stride != 0 where the level is stored */
-  double *d_vert;        /* mapped: vertex planes lv.coef_cz0 .. lv.cz_hi of the stored cell layers (rhs, solution norm) */
+  int mapped;            /* created by pmg_laplace_operator_create_mapped / _curved: lv.geo_stride != 0 where the level is stored */
+  int geo_degree;        /* mapped: the cells' geometry degree k (1 = trilinear) */
+  double *d_vert;        /* mapped: node planes k lv.coef_cz0 .. k lv.cz_hi of the stored cell layers (rhs, solution norm) */
   pmg_vector *dinv;      /* explicit inverse diagonal once compute_diagonal() ran */
   pmg_vector *cg_ws[4];  /* CG work vectors r, z, p, Ap: created by the first pmg_cg_solve, kept until destroy */
 };

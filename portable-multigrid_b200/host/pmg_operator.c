@@ -45,9 +45,10 @@ static int setup_coefficient(pmg_operator *op)
 }
 
 /* Mapped geometry (SURVEY.md row f4): the six entries of G_q = w_q a(x_q) |det J_q| J_q^-1 J_q^-T of every quadrature point
-   of the locally stored cell layers, computed on the device from the trilinear maps of the cells (csrc/pmg_apply_geo.cu)
-   and streamed by the tensor variant of the variable-coefficient kernel.  Only the vertex planes of the stored layers are
-   uploaded; a cell with det J <= 0 at a Gauss point or a non-finite vertex rejects the mesh. */
+   of the locally stored cell layers, computed on the device from the cells' maps (csrc/pmg_apply_geo.cu) -- trilinear
+   (geometry degree 1) or the degree-k Lagrange interpolant through (k+1)^3 nodes (curved cells, MappingQ(k)) -- and
+   streamed by the tensor variant of the variable-coefficient kernel.  Only the node planes of the stored layers are
+   uploaded; a cell with det J <= 0 at a Gauss point or a non-finite node rejects the mesh. */
 static int geo_diagonal(pmg_operator *op)
 {
   const int n1 = op->degree + 1;
@@ -57,8 +58,9 @@ static int geo_diagonal(pmg_operator *op)
   return pmgk_geo_fill_dinv(&op->lv, Sq, G, SG, op->dinv->d, op->ctx->stream);
 }
 
-static int setup_geometry(pmg_operator *op, const double *vertices)
+static int setup_geometry(pmg_operator *op, const double *nodes)
 {
+  const int k = op->geo_degree;
   pmgk_level *lv = &op->lv;
   double gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
   pmg_fe_shape_tables(op->degree, lv->Sq, lv->Dco, NULL, gq, gw);
@@ -72,26 +74,27 @@ static int setup_geometry(pmg_operator *op, const double *vertices)
     return PMG_ERR_NOMEM;
   }
   lv->coef = op->d_coef;
-  /* vertex planes coef_cz0 .. cz_hi of the stored cell layers, and one error word */
-  const size_t vplane = (size_t)(lv->nx + 1) * (lv->ny + 1) * 3;
-  const size_t nv = vplane * (size_t)(lv->cz_hi - lv->coef_cz0 + 1);
+  /* node planes k coef_cz0 .. k cz_hi of the stored cell layers, and one error word */
+  const size_t vplane = (size_t)(lv->nx * (size_t)k + 1) * (lv->ny * (size_t)k + 1) * 3;
+  const size_t nv = vplane * ((size_t)(lv->cz_hi - lv->coef_cz0) * k + 1);
   cudaStream_t st = op->ctx->stream;
   unsigned long long *d_err = NULL, h_err = 0;
   int rc = PMG_OK;
   if (cudaMalloc((void **)&op->d_vert, sizeof(double) * nv + sizeof(unsigned long long)) != cudaSuccess) {
-    pmg_set_error("cudaMalloc of %lld vertex coordinates failed", (long long)nv);
+    pmg_set_error("cudaMalloc of %lld node coordinates failed", (long long)nv);
     return PMG_ERR_NOMEM;
   }
   d_err = (unsigned long long *)(op->d_vert + nv);
-  if (cudaMemcpyAsync(op->d_vert, vertices + vplane * lv->coef_cz0, sizeof(double) * nv, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+  if (cudaMemcpyAsync(op->d_vert, nodes + vplane * k * lv->coef_cz0, sizeof(double) * nv, cudaMemcpyHostToDevice, st) != cudaSuccess ||
       cudaMemsetAsync(d_err, 0xFF, sizeof(unsigned long long), st) != cudaSuccess) rc = PMG_ERR_CUDA;
-  if (rc == PMG_OK) rc = pmgk_geo_fill(lv, op->coefficient, op->d_vert, gq, gw, op->d_coef, d_err, st);
+  if (rc == PMG_OK) rc = pmgk_geo_fill(lv, k, op->coefficient, op->d_vert, gq, gw, op->d_coef, d_err, st);
   if (rc == PMG_OK && cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
-  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* vertices and h_err are pageable */
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* nodes and h_err are pageable */
   if (rc != PMG_OK) return rc;
   if (h_err != ~0ull) {
     const long long c = (long long)h_err, cx = c % lv->nx, cy = c / lv->nx % lv->ny, cz = c / ((long long)lv->nx * lv->ny);
-    pmg_set_error("mapped mesh: cell %lld = (%lld, %lld, %lld) has det J <= 0 at a Gauss point or a non-finite vertex", c, cx, cy, cz);
+    pmg_set_error("mapped mesh: cell %lld = (%lld, %lld, %lld) has det J <= 0 at a Gauss point or a non-finite %s", c, cx, cy, cz,
+                  k == 1 ? "vertex" : "node");
     return PMG_ERR_ARG;
   }
   PMG_CHECK(geo_diagonal(op));
@@ -99,8 +102,9 @@ static int setup_geometry(pmg_operator *op, const double *vertices)
   return PMG_OK;
 }
 
+/* nodes: NULL (the box), or the mesh's geometry support points of geometry degree k (k = 1: the vertices) */
 static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz, unsigned faces, int coefficient,
-                           const double *vertices, pmg_operator **out)
+                           const double *nodes, int k, pmg_operator **out)
 {
   if (!ctx || !out || nx < 1 || ny < 1 || nz < 1) { pmg_set_error("operator_create: bad arguments"); return PMG_ERR_ARG; }
   if (dim != 2 && dim != 3) { pmg_set_error("dim = %d: the reference instantiates dim = 2 and dim = 3", dim); return PMG_ERR_UNSUPPORTED; }
@@ -112,7 +116,8 @@ static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny
   pmg_operator *op = (pmg_operator *)calloc(1, sizeof(*op));
   if (!op) return PMG_ERR_NOMEM;
   op->ctx = ctx; op->dim = dim; op->degree = degree; op->coefficient = coefficient; op->faces = faces & PMG_ALL_FACES;
-  op->mapped = vertices != NULL;
+  op->mapped = nodes != NULL;
+  op->geo_degree = nodes ? k : 0;
   PMG_CHECK(pmg_layout_make(ctx, dim, degree, nx, ny, nz, &op->lay));
   pmgk_level *lv = &op->lv;
   lv->dim = dim;
@@ -139,8 +144,8 @@ static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny
   lv->dinv_vec = NULL;
   const char *tv = getenv("PMG_TILE_VARIANT");
   lv->tile_variant = tv ? atoi(tv) : 0;
-  if (vertices) {
-    const int rc = setup_geometry(op, vertices);
+  if (nodes) {
+    const int rc = setup_geometry(op, nodes);
     if (rc != PMG_OK) { pmg_laplace_operator_destroy(op); return rc; }
   } else if (coefficient != 0) {
     const int rc = setup_coefficient(op);
@@ -153,14 +158,25 @@ static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny
 int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz,
                                 unsigned faces, int coefficient, pmg_operator **out)
 {
-  return operator_create(ctx, dim, degree, nx, ny, nz, faces, coefficient, NULL, out);
+  return operator_create(ctx, dim, degree, nx, ny, nz, faces, coefficient, NULL, 0, out);
 }
 
 int pmg_laplace_operator_create_mapped(pmg_context *ctx, int degree, int nx, int ny, int nz, unsigned faces, int coefficient,
                                        const double *vertices, pmg_operator **out)
 {
   if (!vertices) { pmg_set_error("operator_create_mapped: no vertices"); return PMG_ERR_ARG; }
-  return operator_create(ctx, 3, degree, nx, ny, nz, faces, coefficient, vertices, out);
+  return operator_create(ctx, 3, degree, nx, ny, nz, faces, coefficient, vertices, 1, out);
+}
+
+int pmg_laplace_operator_create_curved(pmg_context *ctx, int degree, int geometry_degree, int nx, int ny, int nz, unsigned faces,
+                                       int coefficient, const double *nodes, pmg_operator **out)
+{
+  if (geometry_degree < 1 || geometry_degree > PMG_MAX_DEGREE) {
+    pmg_set_error("geometry degree %d outside 1..%d", geometry_degree, PMG_MAX_DEGREE);
+    return PMG_ERR_UNSUPPORTED;
+  }
+  if (!nodes) { pmg_set_error("operator_create_curved: no nodes"); return PMG_ERR_ARG; }
+  return operator_create(ctx, 3, degree, nx, ny, nz, faces, coefficient, nodes, geometry_degree, out);
 }
 
 int pmg_laplace_operator_destroy(pmg_operator *op)
@@ -399,7 +415,7 @@ static int mapped_rhs(const pmg_operator *op, pmg_vector *rhs)
   double *W = NULL;
   const int64_t n = pmgk_var_coef_doubles(lv);
   if (cudaMallocAsync((void **)&W, sizeof(double) * (size_t)(n > 0 ? n : 1), st) != cudaSuccess) return PMG_ERR_NOMEM;
-  int rc = pmgk_geo_rhs(lv, op->d_vert, S, gq, gw, W, rhs->d, st);
+  int rc = pmgk_geo_rhs(lv, op->geo_degree, op->d_vert, S, gq, gw, W, rhs->d, st);
   cudaFreeAsync(W, st);
   if (rc != PMG_OK) return rc;
   return pmg_halo_update(op->ctx, &op->lay, rhs->d);
@@ -422,7 +438,7 @@ static int mapped_norm(const pmg_operator *op, const pmg_vector *u, double *norm
     double *sums = NULL;
     PMG_CHECK(pmg_halo_update(ctx, &u->lay, u->d));
     if (cudaMallocAsync((void **)&sums, sizeof(double) * (size_t)(ncells > 0 ? ncells : 1), ctx->stream) != cudaSuccess) return PMG_ERR_NOMEM;
-    int rc = pmgk_geo_norm_cells(lv, op->d_vert, E, g, w, u->d, sums, ctx->stream);
+    int rc = pmgk_geo_norm_cells(lv, op->geo_degree, op->d_vert, E, g, w, u->d, sums, ctx->stream);
     if (rc == PMG_OK) rc = pmgk_sum(sums, ncells, ctx->scalars, ctx->work, ctx->stream);
     cudaFreeAsync(sums, ctx->stream);
     if (rc != PMG_OK) return rc;

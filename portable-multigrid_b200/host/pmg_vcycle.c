@@ -448,6 +448,13 @@ int pmg_host_pencil(int degree, double *M, double *K)
   return PMG_OK;
 }
 
+int pmg_host_support_points(int degree, double *x)
+{
+  if (degree < 1 || degree > PMG_MAX_DEGREE || !x) return PMG_ERR_ARG;
+  pmg_fe_gll(degree + 1, x);
+  return PMG_OK;
+}
+
 int pmg_host_prolongation_1d(int kind, int degree_coarse, int degree_fine, double *P)
 {
   if (!P || degree_coarse < 1 || degree_coarse > PMG_MAX_DEGREE) return PMG_ERR_ARG;

@@ -15,6 +15,7 @@ LIB_PATH = os.path.normpath(os.path.join(_HERE, "..", "..", "lib", "libpmg.so"))
 
 PMG_ALL_FACES = 0x3F
 PMG_INVALID_DEGREE = -1
+PMG_MAX_DEGREE = 9
 _dp = C.POINTER(C.c_double)
 _vp = C.c_void_p
 
@@ -219,21 +220,39 @@ class Vector:
 class LaplaceOperator:
     """Portable::LaplaceOperator (reference include/operators/portable_laplace_operator.h:383-461)."""
 
-    def __init__(self, ctx, degree, n, dirichlet_faces=PMG_ALL_FACES, dim=3, coefficient=0, vertices=None):
+    def __init__(self, ctx, degree, n, dirichlet_faces=PMG_ALL_FACES, dim=3, coefficient=0, vertices=None, nodes=None,
+                 geometry_degree=None):
         """vertices: None (the unit cube cut into equal boxes) or the (nx+1)(ny+1)(nz+1) mesh vertices of a deformed
-        structured mesh, shape (nz+1, ny+1, nx+1, 3) or flat in that order (pmg_laplace_operator_create_mapped); 3-D only."""
+        structured mesh, shape (nz+1, ny+1, nx+1, 3) or flat in that order (pmg_laplace_operator_create_mapped); 3-D only.
+        nodes: instead of vertices, the (nx k+1)(ny k+1)(nz k+1) geometry support points of curved cells of degree
+        k = geometry_degree (mesh_nodes; pmg_laplace_operator_create_curved), shape (nz k+1, ny k+1, nx k+1, 3) or flat;
+        geometry_degree None: the k the array's size implies."""
         if isinstance(n, int):
             n = (n,) * dim
         n = tuple(n) + (1,) * (3 - len(n))  # dim = 2: (nx, ny); the C-ABI ignores nz
         self.ctx, self.degree, self.ncells, self.dim = ctx, degree, tuple(n), dim
         self.h = _vp()
         self.vertices = None
-        if vertices is None:
+        self.nodes, self.geometry_degree = None, None
+        if vertices is None and nodes is None:
             _ck(lib().pmg_laplace_operator_create(ctx.h, C.c_int(dim), C.c_int(degree), C.c_int(n[0]), C.c_int(n[1]),
                                                   C.c_int(n[2]), C.c_uint(dirichlet_faces), C.c_int(coefficient), C.byref(self.h)))
             return
+        if vertices is not None and nodes is not None:
+            raise PmgError(-1, "vertices= and nodes= are mutually exclusive")
         if dim != 3:
             raise PmgError(-3, "the mapped operator is 3-D only (dim = %d)" % dim)
+        if nodes is not None:
+            v = np.ascontiguousarray(nodes, dtype=np.float64).reshape(-1)
+            k = geometry_degree if geometry_degree is not None else _geometry_degree_of(v.size, n)
+            if 1 <= k <= PMG_MAX_DEGREE and v.size != 3 * _n_nodes(n, k):
+                raise PmgError(-1, "nodes: %d values for %d x %d x %d cells of geometry degree %d, need 3 (nx k+1)(ny k+1)(nz k+1)"
+                               % (v.size, *n, k))
+            _ck(lib().pmg_laplace_operator_create_curved(ctx.h, C.c_int(degree), C.c_int(k), C.c_int(n[0]), C.c_int(n[1]),
+                                                         C.c_int(n[2]), C.c_uint(dirichlet_faces), C.c_int(coefficient),
+                                                         _np_ptr(v), C.byref(self.h)))
+            self.nodes, self.geometry_degree = v.reshape(n[2] * k + 1, n[1] * k + 1, n[0] * k + 1, 3), k
+            return
         v = np.ascontiguousarray(vertices, dtype=np.float64).reshape(-1)
         if v.size != 3 * (n[0] + 1) * (n[1] + 1) * (n[2] + 1):
             raise PmgError(-1, "vertices: %d values for %d x %d x %d cells, need 3 (nx+1)(ny+1)(nz+1)" % (v.size, *n))
@@ -420,15 +439,27 @@ def cg_solve(A, x, b, precond=None, max_iterations=None, tolerance=None, rel_tol
 
 
 def build_hierarchy(ctx, levels, pre=2, post=2, degree=5, smoothing_range=15.0, eig_cg_n_iterations=10,
-                    coarse_range=1e-3, faces=PMG_ALL_FACES, coefficient=0, dim=3, vertices=None):
+                    coarse_range=1e-3, faces=PMG_ALL_FACES, coefficient=0, dim=3, vertices=None, mapping=None,
+                    geometry_degree=None):
     """levels: list of (degree, n_cells) coarse -> fine; consecutive levels must be related by one
     global refinement (h) or a degree change on the same mesh (p).  Smoother parameters as in the
     reference drivers (program.cc:267-279).  coefficient = 1: every level discretises -div(a grad u) with
     a = 1/(0.05 + 2|x|^2) at its own quadrature points (BASELINE config 5).  vertices: the finest mesh's vertices
-    (LaplaceOperator); a coarser mesh takes every 2^k-th vertex in each direction (nested meshes), p-levels share them."""
-    ops = [LaplaceOperator(ctx, p, n, faces, dim=dim, coefficient=coefficient,
-                           vertices=None if vertices is None else mesh_vertices_coarsened(vertices, levels[-1][1], n))
-           for (p, n) in levels]
+    (LaplaceOperator); a coarser mesh takes every 2^k-th vertex in each direction (nested meshes), p-levels share them.
+    mapping: instead of vertices, a map of the unit cube (mesh_nodes); every level gets curved cells interpolating it,
+    of the level's FE degree (MappingQ(p) on every level) or of geometry_degree when that is given."""
+    if vertices is not None and mapping is not None:
+        raise PmgError(-1, "vertices= and mapping= are mutually exclusive")
+
+    def level_op(p, n):
+        if mapping is not None:
+            k = p if geometry_degree is None else geometry_degree
+            return LaplaceOperator(ctx, p, n, faces, dim=dim, coefficient=coefficient, nodes=mesh_nodes(mapping, n, k),
+                                   geometry_degree=k)
+        return LaplaceOperator(ctx, p, n, faces, dim=dim, coefficient=coefficient,
+                               vertices=None if vertices is None else mesh_vertices_coarsened(vertices, levels[-1][1], n))
+
+    ops = [level_op(p, n) for (p, n) in levels]
     transfers = []
     for l in range(1, len(levels)):
         if levels[l][0] == levels[l - 1][0]:
@@ -466,6 +497,41 @@ def mesh_vertices_uniform(n, box=(1.0, 1.0, 1.0)):
     n = (n,) * 3 if isinstance(n, int) else tuple(n)
     z, y, x = np.meshgrid(*[np.arange(n[d] + 1) * (box[d] / n[d]) for d in (2, 1, 0)], indexing="ij")
     return np.ascontiguousarray(np.stack([x, y, z], axis=-1))
+
+
+def _n_nodes(n, k):
+    return (n[0] * k + 1) * (n[1] * k + 1) * (n[2] * k + 1)
+
+
+def _geometry_degree_of(size, n):
+    """the geometry degree k >= 1 with 3 (nx k+1)(ny k+1)(nz k+1) = size; PmgError(-1) when there is none"""
+    k = 1
+    while 3 * _n_nodes(n, k) < size:
+        k += 1
+    if 3 * _n_nodes(n, k) != size:
+        raise PmgError(-1, "nodes: %d values fit no geometry degree for %d x %d x %d cells" % (size, *n))
+    return k
+
+
+def host_support_points(k):
+    """the k + 1 Gauss-Lobatto points of [0, 1] the nodes of a curved cell of geometry degree k sit at"""
+    x = np.zeros(k + 1)
+    _ck(lib().pmg_host_support_points(C.c_int(k), _np_ptr(x)))
+    return x
+
+
+def mesh_nodes(mapping, n, k):
+    """Geometry support points of a structured mesh of n cells (int or (nx, ny, nz)) on the image of the unit cube under
+    mapping(X, Y, Z) -> array (..., 3): the map evaluated at the degree-k Gauss-Lobatto grid of every cell
+    (host_support_points), shape (nz k+1, ny k+1, nx k+1, 3) -- the nodes= array of LaplaceOperator."""
+    n = (n,) * 3 if isinstance(n, int) else tuple(n)
+    s = host_support_points(k)
+    t = [np.concatenate([(c + s[:-1]) / nd for c in range(nd)] + [[1.0]]) for nd in n]
+    Z, Y, X = np.meshgrid(t[2], t[1], t[0], indexing="ij")
+    out = np.ascontiguousarray(np.asarray(mapping(X, Y, Z), dtype=np.float64))
+    if out.shape != X.shape + (3,):
+        raise PmgError(-1, "mapping returned shape %s for points of shape %s, need (..., 3)" % (out.shape, X.shape))
+    return out
 
 
 def host_fastdiag_tables(p):
