@@ -152,7 +152,8 @@ def test_residual_and_vector_ops(pmg, ctx, oracle):
     assert du.size() == N and du.locally_owned_size() == N
 
 
-@pytest.mark.parametrize("p,nc", [(1, (3, 4, 2)), (2, (3, 2, 4)), (3, (2, 3, 2)), (4, (2, 2, 3)), (5, (2, 1, 2))])
+@pytest.mark.parametrize("p,nc", [(1, (3, 4, 2)), (2, (3, 2, 4)), (3, (2, 3, 2)), (4, (2, 2, 3)), (5, (2, 1, 2)),
+                                  (6, (2, 1, 2)), (7, (1, 2, 1)), (8, (2, 1, 1)), (9, (1, 1, 2))])
 def test_h_transfer_matches_oracle(p, nc, pmg, ctx, oracle):
     nf = tuple(2 * c for c in nc)
     mc, mf = oracle.MatrixFree(3, p, nc), oracle.MatrixFree(3, p, nf)
@@ -172,7 +173,7 @@ def test_h_transfer_matches_oracle(p, nc, pmg, ctx, oracle):
     assert rel_l2(dc2.export_host(), ref) <= 1e-13
 
 
-@pytest.mark.parametrize("pc,pf", [(1, 2), (2, 4), (1, 4), (3, 4), (2, 3), (4, 7), (6, 7), (4, 8)])
+@pytest.mark.parametrize("pc,pf", [(1, 2), (2, 4), (1, 4), (3, 4), (2, 3), (4, 7), (6, 7), (4, 8), (4, 9), (3, 7), (3, 6), (2, 5), (1, 3)])
 def test_p_transfer_matches_oracle(pc, pf, pmg, ctx, oracle):
     n = (3, 2, 3)
     mc, mf = oracle.MatrixFree(3, pc, n), oracle.MatrixFree(3, pf, n)

@@ -125,12 +125,14 @@ def interpolation_1d(p_from, n_from, p_to, n_to):
     x_to = dof_grid(p_to, [n_to])[0]
     Nf = n_from * p_from + 1
     M = np.zeros((len(x_to), Nf))
-    basis = lagrange(gll_nodes(p_from))
+    g = gll_nodes(p_from)
     for r, x in enumerate(x_to):
         c = min(int(np.floor(x * n_from + 1e-12)), n_from - 1)
         xi = x * n_from - c
-        for i, b in enumerate(basis):
-            M[r, c * p_from + i] = Pn.polyval(xi, b)  # a vertex of the `from` mesh is found in one cell only: assigned, not summed
+        for i in range(p_from + 1):
+            # product form of the Lagrange polynomial: monomial coefficients lose ~1e-11 to cancellation at degree 9
+            v = np.prod([(xi - g[j]) / (g[i] - g[j]) for j in range(p_from + 1) if j != i])
+            M[r, c * p_from + i] = v  # a vertex of the `from` mesh is found in one cell only: assigned, not summed
     return M
 
 
@@ -174,17 +176,29 @@ def test_variable_coefficient_operator_matches_dense_assembly(p, n, oracle):
     assert rel_l2(mf.compute_diagonal(), 1.0 / np.diag(A)) < 1e-12
 
 
-@pytest.mark.parametrize("kind,pc,pf,n", [("h", 1, 1, (2, 2, 1)), ("h", 2, 2, (2, 1, 2)), ("h", 3, 3, (1, 2, 1)), ("h", 4, 4, (2, 2)),
-                                          ("p", 1, 2, (2, 3, 2)), ("p", 2, 4, (2, 2, 1)), ("p", 1, 3, (3, 2)), ("p", 3, 7, (2, 2)), ("p", 2, 5, (1, 2, 2))])
-def test_transfers_match_dense_interpolation(kind, pc, pf, n, oracle):
+_TRANSFER_CASES = [("h", 1, 1, (2, 2, 1)), ("h", 2, 2, (2, 1, 2)), ("h", 3, 3, (1, 2, 1)), ("h", 4, 4, (2, 2)),
+                   ("p", 1, 2, (2, 3, 2)), ("p", 2, 4, (2, 2, 1)), ("p", 1, 3, (3, 2)), ("p", 3, 7, (2, 2)), ("p", 2, 5, (1, 2, 2))]
+# natural faces (the oracle's transfers skip constrained dofs by face) and the degrees 5..9 of the GPU transfers' generic kernels:
+# h Q5..Q9, and the p pairs of the halving hierarchies and of the largest degree gaps
+_TRANSFER_CASES_FACES = [(kind, pc, pf, n, faces) for (kind, pc, pf, n) in
+                         [("h", 1, 1, (2, 1, 2)), ("h", 2, 2, (1, 2, 2)), ("h", 5, 5, (1, 2, 1)), ("h", 6, 6, (2, 1, 1)),
+                          ("h", 7, 7, (1, 1, 2)), ("h", 8, 8, (1, 2, 1)), ("h", 9, 9, (1, 1, 1)), ("p", 1, 2, (2, 1, 2)),
+                          ("p", 1, 3, (1, 2, 1)), ("p", 2, 5, (2, 1, 1)), ("p", 3, 6, (1, 1, 2)), ("p", 3, 7, (1, 2, 1)),
+                          ("p", 4, 8, (2, 1, 1)), ("p", 4, 9, (1, 1, 2)), ("p", 2, 9, (1, 2, 1)), ("p", 8, 9, (2, 1, 1))]
+                         for faces in (0x00, 0x15, 0x2A, 0x03, 0x30, 0x09)]
+
+
+@pytest.mark.parametrize("kind,pc,pf,n,faces",
+                         [pytest.param(*c, 0x3F if len(c[3]) == 3 else 0x0F, id="%s-%d-%d-n%d" % (*c[:3], i)) for i, c in enumerate(_TRANSFER_CASES)] +
+                         [pytest.param(*c, id="%s-%d-%d-%s-f%02x" % (*c[:3], "x".join(map(str, c[3])), c[4])) for c in _TRANSFER_CASES_FACES])
+def test_transfers_match_dense_interpolation(kind, pc, pf, n, faces, oracle):
     """prolongate_and_add: x_f += Z_f P x_c; restrict_and_add: x_c += Z_c P^T Z_f x_f, P = interpolation between the nested spaces
     (the reference realises Z by zero weights and invalid coarse indices, SURVEY.md section 8a8)."""
     dim = len(n)
     nf = tuple(2 * c for c in n) if kind == "h" else n
-    faces = 0x3F if dim == 3 else 0x0F
     Pd = kron_xyz([interpolation_1d(pc, n[d], pf, nf[d]) for d in range(dim)])
     zc, zf = ~constrained_mask(pc, n, faces), ~constrained_mask(pf, nf, faces)
-    mc, mf = oracle.MatrixFree(dim, pc, n), oracle.MatrixFree(dim, pf, nf)
+    mc, mf = oracle.MatrixFree(dim, pc, n, faces=faces), oracle.MatrixFree(dim, pf, nf, faces=faces)
     t = oracle.Transfer(mc, mf, kind)
     rng = np.random.default_rng(pc + 10 * pf)
     xc, xf = rng.standard_normal(mc.n_dofs), rng.standard_normal(mf.n_dofs)
