@@ -134,6 +134,26 @@ int pmg_laplace_operator_vmult_host(const pmg_operator *op, double *dst_host, co
 int pmg_laplace_operator_assemble_rhs(const pmg_operator *op, pmg_vector *rhs);
 int pmg_laplace_operator_solution_norm(const pmg_operator *op, const pmg_vector *u, double *norm);
 
+/* ---- problem data from the caller: f and g as dof vectors of the operator's layout (values at the dof support points) ----
+   The workflow of the reference's matrix-free drivers with inhomogeneous data: fill f and g (e.g. with the coordinates from
+   support_points, pmg_vector_import_host / _import_owned), assemble_rhs_data, solve A u0 = rhs with pmg_cg_solve and the
+   V-cycle (rhs has zero constrained rows, like assemble_rhs), then distribute(u0, g); solution_norm then includes the
+   boundary values.  Every call below returns PMG_ERR_ARG for a vector of another layout. */
+/* Coordinates of the dof support points (FE_Q(degree) Gauss-Lobatto points mapped by the cell's geometry) on all stored
+   planes, ghosts included; z must be NULL for dim = 2 (else PMG_ERR_UNSUPPORTED).  Box: the Gauss-Lobatto grid of the unit
+   cube; mapped: the trilinear map; curved: the degree-k map evaluated at the degree-p Gauss-Lobatto points (k = degree:
+   the nodes themselves). */
+int pmg_laplace_operator_support_points(const pmg_operator *op, pmg_vector *x, pmg_vector *y, pmg_vector *z);
+/* rhs = M f_h - A_free g_D on unconstrained rows, 0 on constrained rows (VectorTools::create_right_hand_side of the nodal
+   interpolant f_h = sum_j f_j phi_j, interpolate_boundary_values + AffineConstraints, program.cc:163-187, 289-334).
+   M: the mass matrix with QGauss(p+1) over the (mapped) cells.  A_free: the operator (with its coefficient and geometry)
+   without Dirichlet masking.  g_D: g on constrained dofs, 0 elsewhere; only the constrained entries of g are read.
+   f == NULL: no volume term; g == NULL: homogeneous.  rhs must differ from f and g.  The ghost planes of rhs are current
+   on return. */
+int pmg_laplace_operator_assemble_rhs_data(const pmg_operator *op, pmg_vector *rhs, const pmg_vector *f, const pmg_vector *g);
+/* u_c = g_c on every constrained dof of the stored planes, other entries untouched (AffineConstraints::distribute, :361) */
+int pmg_laplace_operator_distribute(const pmg_operator *op, pmg_vector *u, const pmg_vector *g);
+
 /* ---- LinearAlgebra::distributed::Vector subset used on the path (SURVEY.md a11) ---- */
 int pmg_vector_destroy(pmg_vector *v);
 int pmg_vector_size(const pmg_vector *v, int64_t *global_size);

@@ -109,6 +109,14 @@ int pmgk_geo_rhs(const pmgk_level *lv, int k, const double *vert, const double *
    vector, ghosts current */
 int pmgk_geo_norm_cells(const pmgk_level *lv, int k, const double *vert, const double *E, const double *gq, const double *gw,
                         const double *u, double *cell_sums, void *stream);
+/* load vector of the nodal interpolant f_h = sum_j f_j phi_j on the mapped mesh, b_i = sum_cells sum_q phi_i(x_q) f_h(x_q)
+   w_q |det J_q| (QGauss(p+1)), on all stored planes as pmgk_geo_rhs (constrained rows 0, ghost planes the stored cells' part):
+   f: local vector of dof values, ghosts current; everything else as pmgk_geo_rhs */
+int pmgk_geo_rhs_f(const pmgk_level *lv, int k, const double *vert, const double *S, const double *gq, const double *gw,
+                   const double *f, double *W, double *rhs, void *stream);
+/* coordinates of the dof support points on all stored planes of the mapped mesh: the cell's map (k, vert as pmgk_geo_fill)
+   at the degree-p Gauss-Lobatto points; x, y, z: local vectors */
+int pmgk_geo_support_points(const pmgk_level *lv, int k, const double *vert, double *x, double *y, double *z, void *stream);
 
 /* inverse diagonal as an explicit vector (LaplaceOperator::compute_diagonal, :752-917) */
 int pmgk_fill_dinv(const pmgk_level *lv, double *dinv, void *stream);
@@ -134,6 +142,11 @@ int pmgk_scalar_div(double *out, const double *num, const double *den, void *str
 /* out[(z * Ny + y) * Nx + x] = lx[x] * ly[y] * lz[z] over nz local planes (lx, ly, lz device arrays): tensor-product
    load vector of the drivers' right-hand side (program.cc:289-334) */
 int pmgk_outer3(double *out, const double *lx, const double *ly, const double *lz, int Nx, int Ny, int nz, void *stream);
+/* masked vector kernels on all stored planes of a level; "constrained" is the face-bitmask test of the apply kernels (lv->faces):
+   out_i = 0 on constrained rows, a x_i + b y_i elsewhere (y may be NULL: a x_i) */
+int pmgk_masked_axpby(const pmgk_level *lv, double *out, double a, const double *x, double b, const double *y, void *stream);
+/* out_i = src_i on constrained rows; elsewhere 0 (zero_free != 0) or out_i unchanged (zero_free = 0) */
+int pmgk_constrained_copy(const pmgk_level *lv, double *out, const double *src, int zero_free, void *stream);
 /* x_i = ((first_global + i) mod 11), Chebyshev eigenvalue-estimate start vector */
 int pmgk_set_mod11(double *x, int64_t first_global, int64_t n, void *stream);
 

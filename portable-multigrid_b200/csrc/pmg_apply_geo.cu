@@ -353,6 +353,143 @@ __global__ void k_curved_norm_cells(const __grid_constant__ CurvedTables t, int 
   }
 }
 
+// ---- problem data from the caller: load vector of a nodal f, support points ------------------------------------------
+// W *= f_h at the quadrature points of the stored cell layers [cz_min, cz_max): f_h = sum_j f_j phi_j interpolated from the
+// cell's (p+1)^3 dofs to its (p+1)^3 Gauss points by sum factorisation with S[q][i] = phi_i(x_q) (x, then y, then z); one
+// thread per cell, W in the layout of one G grid, f a local vector with current ghosts
+template <int P>
+__global__ void k_geo_mul_f(const __grid_constant__ GeoTables t, int nx, int ny, int Nx, int Ny, int z0, int cz_min, int cz_max,
+                            const double *__restrict__ f, double *W)
+{
+  constexpr int N1 = P + 1;
+  const double *S = t.a;
+  const int Qx = nx * N1;
+  const int64_t Qplane = (int64_t)Qx * (ny * N1);
+  const int64_t ncells = (int64_t)nx * ny * (cz_max - cz_min);
+  for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < ncells; c += (int64_t)gridDim.x * blockDim.x) {
+    const int cx = (int)(c % nx), cy = (int)(c / nx % ny), lcz = (int)(c / ((int64_t)nx * ny)), cz = cz_min + lcz;
+    double t1[N1][N1][N1]; // [k][j][qx]
+    for (int k = 0; k < N1; ++k)
+      for (int j = 0; j < N1; ++j) {
+        const double *row = f + ((int64_t)(cz * P + k - z0) * Ny + cy * P + j) * Nx + cx * P;
+        for (int a = 0; a < N1; ++a) {
+          double s = 0.0;
+          for (int i = 0; i < N1; ++i) s += S[a * N1 + i] * row[i];
+          t1[k][j][a] = s;
+        }
+      }
+    double *cw = W + (int64_t)lcz * N1 * Qplane + (int64_t)(cy * N1) * Qx + cx * N1;
+    for (int b = 0; b < N1; ++b) {
+      double t2[N1][N1]; // [k][qx] at qy = b
+      for (int k = 0; k < N1; ++k)
+        for (int a = 0; a < N1; ++a) {
+          double s = 0.0;
+          for (int j = 0; j < N1; ++j) s += S[b * N1 + j] * t1[k][j][a];
+          t2[k][a] = s;
+        }
+      for (int m = 0; m < N1; ++m)
+        for (int a = 0; a < N1; ++a) {
+          double s = 0.0;
+          for (int k = 0; k < N1; ++k) s += S[m * N1 + k] * t2[k][a];
+          cw[m * Qplane + (int64_t)b * Qx + a] *= s;
+        }
+    }
+  }
+}
+
+// The cell a dof of the stored planes is evaluated in: the lower one at a cell boundary (the last cell at the upper end), in z
+// the stored cell layers [cz_min, cz_max).  At a cell boundary the 1-D weights are exactly 0 and 1, so every cell that holds
+// the dof gives the same bits, on every rank.
+__device__ __forceinline__ void support_cell(int g, int P, int c_max, int *c, int *i)
+{
+  int cc = g / P;
+  if (cc > c_max - 1) cc = c_max - 1;
+  *c = cc;
+  *i = g - cc * P;
+}
+
+// support points of the trilinear cells: the map x(xi) = sum_c L_c(xi) v_c (the weights of pmg_geo_point) at the degree-P
+// Gauss-Lobatto points s = t.a; one CTA row per stored (z, y) dof line, threads along x
+template <int P>
+__global__ void k_geo_support(const __grid_constant__ GeoTables t, int nx, int ny, int Nx, int Ny, int z0, int nzl, int cz_min,
+                              int cz_max, const double *__restrict__ vert, double *X, double *Y, double *Z)
+{
+  const double *s = t.a;
+  for (int row = blockIdx.x; row < Ny * nzl; row += gridDim.x) {
+    int cy, iy, cz, iz;
+    support_cell(row % Ny, P, ny, &cy, &iy);
+    support_cell(z0 + row / Ny, P, cz_max, &cz, &iz);
+    for (int gx = threadIdx.x; gx < Nx; gx += blockDim.x) {
+      int cx, ix;
+      support_cell(gx, P, nx, &cx, &ix);
+      double v[8][3];
+      geo_load_cell(vert, nx, ny, cx, cy, cz - cz_min, v);
+      const double L[2][3] = {{1.0 - s[ix], 1.0 - s[iy], 1.0 - s[iz]}, {s[ix], s[iy], s[iz]}};
+      double x[3] = {0.0, 0.0, 0.0};
+      for (int c = 0; c < 8; ++c) {
+        const double w = L[c & 1][0] * L[c >> 1 & 1][1] * L[c >> 2][2];
+        for (int d = 0; d < 3; ++d) x[d] += w * v[c][d];
+      }
+      const int64_t o = (int64_t)row * Nx + gx;
+      X[o] = x[0];
+      Y[o] = x[1];
+      Z[o] = x[2];
+    }
+  }
+}
+
+// as k_geo_support for curved cells: the degree-k map (pmg_curved_map) with the tables t at the degree-P Gauss-Lobatto points
+template <int P>
+__global__ void k_curved_support(const __grid_constant__ CurvedTables t, int k, int nx, int ny, int Nx, int Ny, int z0, int nzl,
+                                 int cz_min, int cz_max, const double *__restrict__ nodes, double *X, double *Y, double *Z)
+{
+  const int k1 = k + 1;
+  const int64_t sy = (int64_t)nx * k + 1, sz = sy * ((int64_t)ny * k + 1);
+  for (int row = blockIdx.x; row < Ny * nzl; row += gridDim.x) {
+    int cy, iy, cz, iz;
+    support_cell(row % Ny, P, ny, &cy, &iy);
+    support_cell(z0 + row / Ny, P, cz_max, &cz, &iz);
+    for (int gx = threadIdx.x; gx < Nx; gx += blockDim.x) {
+      int cx, ix;
+      support_cell(gx, P, nx, &cx, &ix);
+      double x[3], J[3][3];
+      pmg_curved_map(curved_cell_node(nodes, nx, ny, k, cx, cy, cz - cz_min), sy, sz, k, t.L + ix * k1, t.dL + ix * k1,
+                     t.L + iy * k1, t.dL + iy * k1, t.L + iz * k1, t.dL + iz * k1, x, J);
+      const int64_t o = (int64_t)row * Nx + gx;
+      X[o] = x[0];
+      Y[o] = x[1];
+      Z[o] = x[2];
+    }
+  }
+}
+
+template <int P>
+int geo_support_points(const pmgk_level *lv, int k, const double *vert, double *x, double *y, double *z, cudaStream_t s)
+{
+  constexpr int N1 = P + 1;
+  if (lv->nzl <= 0) return 0;
+  double gll[N1];
+  pmg_fe_gll(N1, gll);
+  int64_t rows = (int64_t)lv->Ny * lv->nzl;
+  const int64_t cap = (int64_t)pmgk_device_sm_count() * 32;
+  if (rows > cap) rows = cap;
+  if (k == 1) {
+    GeoTables t;
+    for (int i = 0; i < N1; ++i) t.a[i] = gll[i];
+    k_geo_support<P><<<(unsigned)rows, pmg_var_row_threads(lv->Nx), 0, s>>>(t, lv->nx, lv->ny, lv->Nx, lv->Ny, lv->z0, lv->nzl,
+                                                                          lv->coef_cz0, lv->cz_hi, vert, x, y, z);
+  } else {
+    CurvedTables t;
+    double unused_w[N1] = {};
+    curved_tables(k, N1, gll, unused_w, t);
+    k_curved_support<P><<<(unsigned)rows, pmg_var_row_threads(lv->Nx), 0, s>>>(t, k, lv->nx, lv->ny, lv->Nx, lv->Ny, lv->z0, lv->nzl,
+                                                                             lv->coef_cz0, lv->cz_hi, vert, x, y, z);
+  }
+  PMG_CUDA_CHECK(cudaGetLastError());
+  pmg_count_launch(1);
+  return 0;
+}
+
 template <int P>
 int fill_geo(const pmgk_level *lv, int k, int c5, const double *vert, const double *gq, const double *gw, double *geo,
              unsigned long long *err, cudaStream_t s)
@@ -395,9 +532,10 @@ int fill_geo_dinv(const pmgk_level *lv, const double *S2, const double *G2, cons
   return 0;
 }
 
+// f: NULL = the load vector of f = 1; else the dof values of f_h (k_geo_mul_f between the w |det J| grid and the gather)
 template <int P>
-int geo_rhs(const pmgk_level *lv, int k, const double *vert, const double *S, const double *gq, const double *gw, double *W,
-            double *rhs, cudaStream_t s)
+int geo_rhs(const pmgk_level *lv, int k, const double *vert, const double *S, const double *gq, const double *gw, const double *f,
+            double *W, double *rhs, cudaStream_t s)
 {
   constexpr int N1 = P + 1;
   GeoTables t;
@@ -418,6 +556,15 @@ int geo_rhs(const pmgk_level *lv, int k, const double *vert, const double *S, co
     pmg_count_launch(1);
   }
   for (int i = 0; i < N1 * N1; ++i) t.a[i] = S[i];
+  const int64_t ncells = (int64_t)lv->nx * lv->ny * (lv->cz_hi - lv->coef_cz0);
+  if (f && ncells > 0) {
+    int64_t blocks = (ncells + 127) / 128;
+    const int64_t bcap = (int64_t)pmgk_device_sm_count() * 16;
+    if (blocks > bcap) blocks = bcap;
+    k_geo_mul_f<P><<<(unsigned)blocks, 128, 0, s>>>(t, lv->nx, lv->ny, lv->Nx, lv->Ny, lv->z0, lv->coef_cz0, lv->cz_hi, f, W);
+    PMG_CUDA_CHECK(cudaGetLastError());
+    pmg_count_launch(1);
+  }
   rows = (int64_t)lv->Ny * lv->nzl;
   if (rows > cap) rows = cap;
   if (rows <= 0) return 0;
@@ -465,7 +612,34 @@ extern "C" int pmgk_geo_rhs(const pmgk_level *lv, int k, const double *vert, con
   if (k < 1 || k >= PMGK_MAX_N1) return PMG_ERR_UNSUPPORTED;
   switch (lv->degree) {
 #define PMG_GEO_CASE(P, BX, BY, MINB) \
-  case P: return geo_rhs<P>(lv, k, vert, S, gq, gw, W, rhs, (cudaStream_t)stream);
+  case P: return geo_rhs<P>(lv, k, vert, S, gq, gw, NULL, W, rhs, (cudaStream_t)stream);
+#include "pmg_apply_geo_tiles.inc"
+#undef PMG_GEO_CASE
+    default: return PMG_ERR_UNSUPPORTED;
+  }
+}
+
+extern "C" int pmgk_geo_rhs_f(const pmgk_level *lv, int k, const double *vert, const double *S, const double *gq, const double *gw,
+                              const double *f, double *W, double *rhs, void *stream)
+{
+  if (!lv || !vert || !S || !gq || !gw || !f || !W || !rhs) return PMG_ERR_ARG;
+  if (k < 1 || k >= PMGK_MAX_N1) return PMG_ERR_UNSUPPORTED;
+  switch (lv->degree) {
+#define PMG_GEO_CASE(P, BX, BY, MINB) \
+  case P: return geo_rhs<P>(lv, k, vert, S, gq, gw, f, W, rhs, (cudaStream_t)stream);
+#include "pmg_apply_geo_tiles.inc"
+#undef PMG_GEO_CASE
+    default: return PMG_ERR_UNSUPPORTED;
+  }
+}
+
+extern "C" int pmgk_geo_support_points(const pmgk_level *lv, int k, const double *vert, double *x, double *y, double *z, void *stream)
+{
+  if (!lv || !vert || !x || !y || !z) return PMG_ERR_ARG;
+  if (k < 1 || k >= PMGK_MAX_N1) return PMG_ERR_UNSUPPORTED;
+  switch (lv->degree) {
+#define PMG_GEO_CASE(P, BX, BY, MINB) \
+  case P: return geo_support_points<P>(lv, k, vert, x, y, z, (cudaStream_t)stream);
 #include "pmg_apply_geo_tiles.inc"
 #undef PMG_GEO_CASE
     default: return PMG_ERR_UNSUPPORTED;

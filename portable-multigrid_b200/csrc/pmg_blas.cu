@@ -191,7 +191,73 @@ __global__ void k_outer3(double *out, const double *__restrict__ lx, const doubl
     for (int x = threadIdx.x; x < Nx; x += blockDim.x) o[x] = f * lx[x];
   }
 }
+
+// Dirichlet rows of a level (the face-bitmask test of the apply kernels): one CTA row per stored (z, y) line, threads along x.
+// 2-D levels have one plane (Nz = 1) and faces bits 0..3 only, so the same test holds.
+__device__ __forceinline__ bool pmg_row_constrained_yz(int gy, int gz, int Ny, int Nz, unsigned faces)
+{
+  return (gy == 0 && (faces >> 2 & 1u)) || (gy == Ny - 1 && (faces >> 3 & 1u)) || (gz == 0 && (faces >> 4 & 1u)) ||
+         (gz == Nz - 1 && (faces >> 5 & 1u));
+}
+
+// out = 0 on constrained rows, a x + b y elsewhere (y NULL: a x)
+__global__ void k_masked_axpby(double *out, double a, const double *x, double b, const double *y, int Nx, int Ny, int Nz, int z0,
+                               int nzl, unsigned faces)
+{
+  for (int row = blockIdx.x; row < Ny * nzl; row += gridDim.x) {
+    const bool dyz = pmg_row_constrained_yz(row % Ny, z0 + row / Ny, Ny, Nz, faces);
+    const int64_t o = (int64_t)row * Nx;
+    for (int gx = threadIdx.x; gx < Nx; gx += blockDim.x) {
+      const bool dir = dyz || (gx == 0 && (faces & 1u)) || (gx == Nx - 1 && (faces >> 1 & 1u));
+      out[o + gx] = dir ? 0.0 : (y ? a * x[o + gx] + b * y[o + gx] : a * x[o + gx]);
+    }
+  }
+}
+
+// out = src on constrained rows; elsewhere 0 (zero_free) or untouched
+__global__ void k_constrained_copy(double *out, const double *__restrict__ src, int zero_free, int Nx, int Ny, int Nz, int z0, int nzl,
+                                   unsigned faces)
+{
+  for (int row = blockIdx.x; row < Ny * nzl; row += gridDim.x) {
+    const bool dyz = pmg_row_constrained_yz(row % Ny, z0 + row / Ny, Ny, Nz, faces);
+    const int64_t o = (int64_t)row * Nx;
+    for (int gx = threadIdx.x; gx < Nx; gx += blockDim.x) {
+      const bool dir = dyz || (gx == 0 && (faces & 1u)) || (gx == Nx - 1 && (faces >> 1 & 1u));
+      if (dir) out[o + gx] = src[o + gx];
+      else if (zero_free) out[o + gx] = 0.0;
+    }
+  }
+}
+
+// threads per CTA of the kernels that walk one row of Nx dofs
+inline int row_threads(int Nx) { return Nx >= 192 ? 256 : (Nx >= 96 ? 128 : (Nx >= 48 ? 64 : 32)); }
 } // namespace
+
+extern "C" int pmgk_masked_axpby(const pmgk_level *lv, double *out, double a, const double *x, double b, const double *y, void *stream)
+{
+  if (!lv || !out || !x) return PMG_ERR_ARG;
+  if (lv->nzl <= 0) return 0;
+  int64_t rows = (int64_t)lv->Ny * lv->nzl;
+  const int cap = pmgk_device_sm_count() * 32;
+  if (rows > cap) rows = cap;
+  k_masked_axpby<<<(unsigned)rows, row_threads(lv->Nx), 0, (cudaStream_t)stream>>>(out, a, x, b, y, lv->Nx, lv->Ny, lv->Nz, lv->z0,
+                                                                                   lv->nzl, lv->faces);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int pmgk_constrained_copy(const pmgk_level *lv, double *out, const double *src, int zero_free, void *stream)
+{
+  if (!lv || !out || !src) return PMG_ERR_ARG;
+  if (lv->nzl <= 0) return 0;
+  int64_t rows = (int64_t)lv->Ny * lv->nzl;
+  const int cap = pmgk_device_sm_count() * 32;
+  if (rows > cap) rows = cap;
+  k_constrained_copy<<<(unsigned)rows, row_threads(lv->Nx), 0, (cudaStream_t)stream>>>(out, src, zero_free, lv->Nx, lv->Ny, lv->Nz,
+                                                                                       lv->z0, lv->nzl, lv->faces);
+  LAUNCH_CHECK();
+  return 0;
+}
 
 extern "C" int pmgk_outer3(double *out, const double *lx, const double *ly, const double *lz, int Nx, int Ny, int nz, void *stream)
 {
@@ -199,7 +265,7 @@ extern "C" int pmgk_outer3(double *out, const double *lx, const double *ly, cons
   int64_t rows = (int64_t)Ny * nz;
   const int cap = pmgk_device_sm_count() * 32;
   if (rows > cap) rows = cap;
-  k_outer3<<<(unsigned)rows, Nx >= 192 ? 256 : (Nx >= 96 ? 128 : (Nx >= 48 ? 64 : 32)), 0, (cudaStream_t)stream>>>(out, lx, ly, lz, Nx, Ny, nz);
+  k_outer3<<<(unsigned)rows, row_threads(Nx), 0, (cudaStream_t)stream>>>(out, lx, ly, lz, Nx, Ny, nz);
   LAUNCH_CHECK();
   return 0;
 }

@@ -97,8 +97,10 @@ static double arg_double(int argc, char **argv, const char *name, double def)
    --shell 1 solves on the quarter cylindrical shell 1 <= r <= 2, 0 <= theta <= pi/2, 0 <= z <= 1 with Dirichlet conditions
    on r = 1 and r = 2 and natural ones on the other faces (exact solution u = (1 - r^2)/4 + 3 ln r / (4 ln 2),
    ||u||_L2 = 0.14143644722133), --mapping-degree K the geometry degree of the cells of --distort / --shell: 1 (default)
-   trilinear cells, 0 the level's FE degree (MappingQ(p) on every level), K >= 2 curved cells of degree K */
-static int g_coefficient = 0, g_profile = 0, g_dim = 3, g_shell = 0, g_mapping_degree = 1;
+   trilinear cells, 0 the level's FE degree (MappingQ(p) on every level), K >= 2 curved cells of degree K,
+   --manufactured 1 solves -div(grad u) = f, u = g on the Dirichlet faces, for a known smooth u* (manufactured_values) with f
+   and g = u* interpolated at the dof support points, and prints ||u_h - I_h u*||_L2 after the solution norm */
+static int g_coefficient = 0, g_profile = 0, g_dim = 3, g_shell = 0, g_mapping_degree = 1, g_manufactured = 0;
 static double g_tol = 1e-12, g_distort = 0.0;
 static void common_options(int argc, char **argv)
 {
@@ -108,6 +110,58 @@ static void common_options(int argc, char **argv)
   g_distort = arg_double(argc, argv, "--distort", 0.0);
   g_shell = arg_int(argc, argv, "--shell", 0);
   g_mapping_degree = arg_int(argc, argv, "--mapping-degree", 1);
+  g_manufactured = arg_int(argc, argv, "--manufactured", 0);
+}
+
+/* --manufactured 1: u* and f = -laplace(u*).  Cube: u* = cos(pi x) cos(pi y) cos(pi z), f = 3 pi^2 u* (2-D: without the z
+   factor, f = 2 pi^2 u*).  Shell: the radial u* = r^2 + sin(pi r), f = -u'' - u'/r = -4 + pi^2 sin(pi r) - pi cos(pi r) / r;
+   its normal derivative vanishes on the natural faces theta = 0, pi/2 and z = 0, 1, so only r = 1 and r = 2 need g. */
+static void manufactured_values(double x, double y, double z, double *u, double *f)
+{
+  const double pi = 3.14159265358979323846;
+  if (g_shell) {
+    const double r = sqrt(x * x + y * y);
+    *u = r * r + sin(pi * r);
+    *f = -4.0 + pi * pi * sin(pi * r) - pi * cos(pi * r) / r;
+  } else if (g_dim == 2) {
+    *u = cos(pi * x) * cos(pi * y);
+    *f = 2.0 * pi * pi * *u;
+  } else {
+    *u = cos(pi * x) * cos(pi * y) * cos(pi * z);
+    *f = 3.0 * pi * pi * *u;
+  }
+}
+
+/* f and ustar = I_h u* at the support points of A (evaluated on the host, every rank the full vectors), then
+   rhs = M f_h - A_free g_D with g = ustar (pmg_laplace_operator_assemble_rhs_data) */
+static int manufactured_rhs(pmg_operator *A, pmg_vector *rhs, pmg_vector *ustar)
+{
+  if (g_coefficient) {
+    fprintf(stderr, "--manufactured: f is -laplace(u*), the constant-coefficient problem only\n");
+    return PMG_ERR_UNSUPPORTED;
+  }
+  pmg_vector *X[3] = {NULL, NULL, NULL}, *f = NULL;
+  int64_t m = 0;
+  int rc = pmg_laplace_operator_m(A, &m);
+  for (int d = 0; d < 3 && rc == PMG_OK; ++d) rc = pmg_laplace_operator_initialize_dof_vector(A, &X[d]);
+  if (rc == PMG_OK) rc = pmg_laplace_operator_initialize_dof_vector(A, &f);
+  if (rc == PMG_OK) rc = pmg_laplace_operator_support_points(A, X[0], X[1], g_dim == 3 ? X[2] : NULL);
+  double *h = rc == PMG_OK ? (double *)malloc(sizeof(double) * 5 * (size_t)m) : NULL;
+  if (rc == PMG_OK && !h) rc = PMG_ERR_NOMEM;
+  double *hx = h, *hy = h ? h + m : NULL, *hz = h ? h + 2 * m : NULL, *hu = h ? h + 3 * m : NULL, *hf = h ? h + 4 * m : NULL;
+  if (rc == PMG_OK) rc = pmg_vector_export_host(X[0], hx);
+  if (rc == PMG_OK) rc = pmg_vector_export_host(X[1], hy);
+  if (rc == PMG_OK && g_dim == 3) rc = pmg_vector_export_host(X[2], hz);
+  if (rc == PMG_OK) {
+    for (int64_t i = 0; i < m; ++i) manufactured_values(hx[i], hy[i], g_dim == 3 ? hz[i] : 0.0, hu + i, hf + i);
+    rc = pmg_vector_import_host(ustar, hu);
+  }
+  if (rc == PMG_OK) rc = pmg_vector_import_host(f, hf);
+  if (rc == PMG_OK) rc = pmg_laplace_operator_assemble_rhs_data(A, rhs, f, ustar);
+  free(h);
+  for (int d = 0; d < 3; ++d) pmg_vector_destroy(X[d]);
+  pmg_vector_destroy(f);
+  return rc;
 }
 
 /* the level's operator: on the unit cube, or with --distort / --shell on the image of the unit cube's mesh of n^3 cells
@@ -190,10 +244,15 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
   pmg_vcycle *mg;
   CK(pmg_vcycle_create(ops, tr, sm, L, pre, post, &mg));
   pmg_operator *A = ops[L - 1];
-  pmg_vector *rhs, *x;
+  pmg_vector *rhs, *x, *ustar = NULL;
   CK(pmg_laplace_operator_initialize_dof_vector(A, &rhs));
   CK(pmg_laplace_operator_initialize_dof_vector(A, &x));
-  CK(pmg_laplace_operator_assemble_rhs(A, rhs));
+  if (g_manufactured) {
+    CK(pmg_laplace_operator_initialize_dof_vector(A, &ustar));
+    CK(manufactured_rhs(A, rhs, ustar));
+  } else {
+    CK(pmg_laplace_operator_assemble_rhs(A, rhs));
+  }
   double bnorm = 0.0;
   CK(pmg_vector_l2_norm(rhs, &bnorm));
   int64_t n_dofs = 0;
@@ -207,9 +266,16 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
   CK(pmg_sync(ctx));
   const double dt = now_s() - t0;
   RPRINT("  Solver converged in %d iterations.\n", last_step);
+  if (g_manufactured) CK(pmg_laplace_operator_distribute(A, x, ustar)); /* constraints.distribute (program.cc:361) */
   double norm = 0.0;
   CK(pmg_laplace_operator_solution_norm(A, x, &norm));
   RPRINT("  solution norm: %.10g\n", norm);
+  if (g_manufactured) {
+    double err = 0.0;
+    CK(pmg_vector_sadd(ustar, -1.0, 1.0, x)); /* ustar <- u_h - I_h u* */
+    CK(pmg_laplace_operator_solution_norm(A, ustar, &err));
+    RPRINT("  error: ||u_h - I_h u*||_L2 = %.6e\n", err);
+  }
   RPRINT("  [b200] solve time %.3f ms on %d GPU(s), %.3f GDoF/s (DoFs x iterations / time)\n", dt * 1e3, g_world, (double)n_dofs * last_step / dt / 1e9);
   if (g_profile) {
     double ms[MAXL * 4];
@@ -222,6 +288,7 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
     pmg_vector_destroy(z);
   }
   pmg_vector_destroy(rhs); pmg_vector_destroy(x);
+  if (ustar) pmg_vector_destroy(ustar);
   pmg_vcycle_destroy(mg);
   for (int l = 0; l < L; ++l) { pmg_chebyshev_destroy(sm[l]); if (tr[l]) pmg_transfer_destroy(tr[l]); }
   for (int l = 0; l < L; ++l) pmg_laplace_operator_destroy(ops[l]);

@@ -405,19 +405,27 @@ int pmg_laplace_operator_vmult_host(const pmg_operator *op, double *dst_host, co
 /* Mapped mesh: neither the load vector nor the norm factorises.  b_i = sum_cells sum_q phi_i(x_q) w_q |det J_q| (QGauss(p+1),
    constrained rows dropped) as a deterministic per-dof gather over the <= 8 cells of each dof; the ghost planes are then
    refreshed from their owners. */
-static int mapped_rhs(const pmg_operator *op, pmg_vector *rhs)
+/* f: NULL = f = 1, else the dof values of the nodal f_h, ghosts current (the w |det J| grid is multiplied by f_h at the Gauss
+   points before the gather).  The ghost planes of rhs hold the stored cells' part only. */
+static int mapped_load(const pmg_operator *op, pmg_vector *rhs, const pmg_vector *f)
 {
   const pmgk_level *lv = &op->lv;
-  if (!op->lay.active) return PMG_OK;
   double S[PMGK_MAX_N1 * PMGK_MAX_N1], gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
   pmg_fe_shape_tables(op->degree, S, NULL, NULL, gq, gw);
   cudaStream_t st = op->ctx->stream;
   double *W = NULL;
   const int64_t n = pmgk_var_coef_doubles(lv);
   if (cudaMallocAsync((void **)&W, sizeof(double) * (size_t)(n > 0 ? n : 1), st) != cudaSuccess) return PMG_ERR_NOMEM;
-  int rc = pmgk_geo_rhs(lv, op->geo_degree, op->d_vert, S, gq, gw, W, rhs->d, st);
+  int rc = f ? pmgk_geo_rhs_f(lv, op->geo_degree, op->d_vert, S, gq, gw, f->d, W, rhs->d, st)
+             : pmgk_geo_rhs(lv, op->geo_degree, op->d_vert, S, gq, gw, W, rhs->d, st);
   cudaFreeAsync(W, st);
-  if (rc != PMG_OK) return rc;
+  return rc;
+}
+
+static int mapped_rhs(const pmg_operator *op, pmg_vector *rhs)
+{
+  if (!op->lay.active) return PMG_OK;
+  PMG_CHECK(mapped_load(op, rhs, NULL));
   return pmg_halo_update(op->ctx, &op->lay, rhs->d);
 }
 
@@ -504,6 +512,21 @@ int pmg_laplace_operator_assemble_rhs(const pmg_operator *op, pmg_vector *rhs)
    cell mass matrix): ||u_h||^2 = u^T (Mx (x) My (x) Mz) u.  The apply kernel with the 1-D stiffness matrix replaced by
    the mass matrix computes (cx + cy + cz) (M (x) M (x) M) u for the reference-cell M (csrc/pmg_apply_sweep.h), so the norm
    costs one apply and one dot on the device; boundary values of u are part of the norm, hence no Dirichlet faces. */
+/* Box levels: t = (cx + cy + cz) (M (x) M (x) M) u (2-D: (hy/hx + hx/hy) (M (x) M) u) for the reference-cell mass matrix M,
+   on the owned rows: a copy of the level with the 1-D stiffness matrix replaced by the mass matrix, no Dirichlet faces and
+   no coefficient, through the apply kernel after a ghost update of u (csrc/pmg_apply_sweep.h, 2-D csrc/pmg_dim2.cu) */
+static int box_mass_apply(const pmg_operator *op, const pmg_vector *u, double *t)
+{
+  pmg_context *ctx = op->ctx;
+  pmgk_level lv = op->lv;
+  memcpy(lv.Kref, lv.Mref, sizeof(lv.Kref));
+  lv.faces = 0;
+  lv.coef = NULL; /* the mass matrix has no coefficient */
+  lv.tile_variant = 1; /* the line-marching kernel: the cell-tile kernel works in the eigenbasis of the (M, K) pencil */
+  PMG_CHECK(pmg_halo_update(ctx, &u->lay, u->d));
+  return pmgk_apply(&lv, PMGK_APPLY, u->d, NULL, NULL, t, 0.0, 0.0, ctx->stream);
+}
+
 int pmg_laplace_operator_solution_norm(const pmg_operator *op, const pmg_vector *u, double *norm)
 {
   if (!op || !norm) return PMG_ERR_ARG;
@@ -512,17 +535,9 @@ int pmg_laplace_operator_solution_norm(const pmg_operator *op, const pmg_vector 
   pmg_context *ctx = op->ctx;
   pmg_vector *t = NULL;
   PMG_CHECK(pmg_vector_create_layout(ctx, &op->lay, &t));
-  pmgk_level lv = op->lv;
-  memcpy(lv.Kref, lv.Mref, sizeof(lv.Kref));
-  lv.faces = 0;
-  lv.coef = NULL; /* the mass matrix has no coefficient */
-  lv.tile_variant = 1; /* the line-marching kernel: the cell-tile kernel works in the eigenbasis of the (M, K) pencil */
   int rc = PMG_OK;
   double uMu = 0.0;
-  if (op->lay.active) {
-    rc = pmg_halo_update(ctx, &u->lay, u->d);
-    if (rc == PMG_OK) rc = pmgk_apply(&lv, PMGK_APPLY, u->d, NULL, NULL, t->d, 0.0, 0.0, ctx->stream);
-  }
+  if (op->lay.active) rc = box_mass_apply(op, u, t->d);
   if (rc == PMG_OK) rc = pmg_vector_dot(u, t, &uMu);
   pmg_vector_destroy(t);
   if (rc != PMG_OK) return rc;
@@ -534,4 +549,109 @@ int pmg_laplace_operator_solution_norm(const pmg_operator *op, const pmg_vector 
   const double cx = h[1] * h[2] / h[0], cy = h[0] * h[2] / h[1], cz = h[0] * h[1] / h[2];
   *norm = sqrt(fabs(uMu) * (h[0] * h[1] * h[2]) / (cx + cy + cz));
   return PMG_OK;
+}
+
+/* ---- problem data from the caller: support points, load vector of a nodal f with Dirichlet lifting, distribute ----------- */
+/* Coordinates of the dof support points.  Box: the Gauss-Lobatto grid (c + s_i) / n_d of every direction as three outer
+   products of 1-D lines with ones (pmgk_outer3, exact); mapped: the cells' maps at the Gauss-Lobatto points on the device. */
+int pmg_laplace_operator_support_points(const pmg_operator *op, pmg_vector *x, pmg_vector *y, pmg_vector *z)
+{
+  if (!op) return PMG_ERR_ARG;
+  if (op->dim == 2 && z) { pmg_set_error("support_points: the 2-D operator has no z coordinate (pass z = NULL)"); return PMG_ERR_UNSUPPORTED; }
+  PMG_CHECK(check_vec(op, x, "support_points(x)"));
+  PMG_CHECK(check_vec(op, y, "support_points(y)"));
+  if (op->dim == 3) PMG_CHECK(check_vec(op, z, "support_points(z)"));
+  PMG_CHECK(pmg_enter(op->ctx));
+  const pmg_layout *l = &op->lay;
+  if (!l->active) return PMG_OK;
+  cudaStream_t st = op->ctx->stream;
+  if (op->mapped) return pmgk_geo_support_points(&op->lv, op->geo_degree, op->d_vert, x->d, y->d, z->d, st);
+  const int p = op->degree, N[3] = {l->Nx, l->Ny, l->Nz}, nc[3] = {l->nx, l->ny, l->nz};
+  double gll[PMG_MAX_DEGREE + 2];
+  pmg_fe_gll(p + 1, gll);
+  /* host: the lines x, y, z, then ones (as long as the longest line) */
+  const int nmax = N[0] > N[1] ? (N[0] > N[2] ? N[0] : N[2]) : (N[1] > N[2] ? N[1] : N[2]);
+  const size_t nl = (size_t)N[0] + N[1] + N[2] + nmax;
+  double *h = (double *)malloc(sizeof(double) * nl), *d = NULL;
+  if (!h) return PMG_ERR_NOMEM;
+  double *line[3] = {h, h + N[0], h + N[0] + N[1]}, *ones = h + N[0] + N[1] + N[2];
+  line[2][0] = 0.0; /* 2-D: the single plane, no z line */
+  for (int e = 0; e < op->dim; ++e) {
+    for (int c = 0; c < nc[e]; ++c)
+      for (int i = 0; i < p; ++i) line[e][c * p + i] = (c + gll[i]) / nc[e];
+    line[e][N[e] - 1] = 1.0;
+  }
+  for (int i = 0; i < nmax; ++i) ones[i] = 1.0;
+  int rc = PMG_OK;
+  if (cudaMallocAsync((void **)&d, sizeof(double) * nl, st) != cudaSuccess ||
+      cudaMemcpyAsync(d, h, sizeof(double) * nl, cudaMemcpyHostToDevice, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  double *dl[3] = {d, d + N[0], d + N[0] + N[1]}, *d1 = d + N[0] + N[1] + N[2];
+  if (rc == PMG_OK) rc = pmgk_outer3(x->d, dl[0], d1, d1, l->Nx, l->Ny, l->nzl, st);
+  if (rc == PMG_OK) rc = pmgk_outer3(y->d, d1, dl[1], d1, l->Nx, l->Ny, l->nzl, st);
+  if (rc == PMG_OK && z) rc = pmgk_outer3(z->d, d1, d1, dl[2] + l->z0, l->Nx, l->Ny, l->nzl, st);
+  if (d) cudaFreeAsync(d, st);
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* h is pageable */
+  free(h);
+  return rc;
+}
+
+/* rhs = M f_h - A_free g_D on unconstrained rows, 0 on constrained rows (VectorTools::create_right_hand_side of the nodal
+   interpolant and the lifting of AffineConstraints with inhomogeneous Dirichlet values, program.cc:163-187, 289-334).
+   M f_h: box levels through the mass-matrix copy of the level (box_mass_apply) scaled by h_x h_y h_z / (c_x + c_y + c_z);
+   mapped levels through the w |det J| grid times f_h at the Gauss points and the per-dof gather.  The lifting: g_D = g
+   masked to the constrained dofs, its ghost planes refreshed, t = A_free g_D with the level's operator without Dirichlet
+   faces (the plain apply, with the level's coefficient or geometry), rhs = rhs - t on unconstrained rows. */
+int pmg_laplace_operator_assemble_rhs_data(const pmg_operator *op, pmg_vector *rhs, const pmg_vector *f, const pmg_vector *g)
+{
+  if (!op) return PMG_ERR_ARG;
+  PMG_CHECK(check_vec(op, rhs, "assemble_rhs_data(rhs)"));
+  if (f) PMG_CHECK(check_vec(op, f, "assemble_rhs_data(f)"));
+  if (g) PMG_CHECK(check_vec(op, g, "assemble_rhs_data(g)"));
+  if (rhs == f || rhs == g) { pmg_set_error("assemble_rhs_data: rhs must differ from f and g"); return PMG_ERR_ARG; }
+  PMG_CHECK(pmg_enter(op->ctx));
+  pmg_context *ctx = op->ctx;
+  const pmg_layout *l = &op->lay;
+  if (!l->active) return PMG_OK;
+  cudaStream_t st = ctx->stream;
+  pmg_vector *t0 = NULL, *t1 = NULL;
+  PMG_CHECK(pmg_vector_create_layout(ctx, l, &t0));
+  int rc = PMG_OK;
+  if (f && op->mapped) {
+    rc = pmg_halo_update(ctx, &f->lay, f->d);
+    if (rc == PMG_OK) rc = mapped_load(op, rhs, f);
+  } else if (f) {
+    const double *h = op->lv.h;
+    double scale;
+    if (op->dim == 2) scale = (h[0] * h[1]) / (h[1] / h[0] + h[0] / h[1]);
+    else scale = (h[0] * h[1] * h[2]) / (h[1] * h[2] / h[0] + h[0] * h[2] / h[1] + h[0] * h[1] / h[2]);
+    rc = box_mass_apply(op, f, t0->d);
+    if (rc == PMG_OK) rc = pmgk_masked_axpby(&op->lv, rhs->d, scale, t0->d, 0.0, NULL, st);
+  } else {
+    rc = pmgk_set(rhs->d, 0.0, l->n_local, st);
+  }
+  if (rc == PMG_OK && g) {
+    rc = pmg_vector_create_layout(ctx, l, &t1);
+    pmgk_level lv = op->lv;
+    lv.faces = 0;
+    if (rc == PMG_OK) rc = pmgk_constrained_copy(&op->lv, t0->d, g->d, 1, st);
+    if (rc == PMG_OK) rc = pmg_halo_update(ctx, l, t0->d);
+    if (rc == PMG_OK) rc = pmgk_apply(&lv, PMGK_APPLY, t0->d, NULL, NULL, t1->d, 0.0, 0.0, st);
+    if (rc == PMG_OK) rc = pmgk_masked_axpby(&op->lv, rhs->d, 1.0, rhs->d, -1.0, t1->d, st);
+  }
+  if (rc == PMG_OK) rc = pmg_halo_update(ctx, l, rhs->d);
+  pmg_vector_destroy(t0);
+  if (t1) pmg_vector_destroy(t1);
+  return rc;
+}
+
+/* u_c = g_c on the constrained dofs of the stored planes, every other entry untouched (AffineConstraints::distribute,
+   program.cc:361) */
+int pmg_laplace_operator_distribute(const pmg_operator *op, pmg_vector *u, const pmg_vector *g)
+{
+  if (!op) return PMG_ERR_ARG;
+  PMG_CHECK(check_vec(op, u, "distribute(u)"));
+  PMG_CHECK(check_vec(op, g, "distribute(g)"));
+  PMG_CHECK(pmg_enter(op->ctx));
+  if (!op->lay.active || u == g) return PMG_OK;
+  return pmgk_constrained_copy(&op->lv, u->d, g->d, 0, op->ctx->stream);
 }

@@ -325,6 +325,28 @@ class LaplaceOperator:
         _ck(lib().pmg_laplace_operator_solution_norm(self.h, u.h, C.byref(r)))
         return r.value
 
+    def support_points(self):
+        """The dof support points, an (m, dim) array in global lexicographic order (pmg_laplace_operator_support_points)."""
+        vs = [self.initialize_dof_vector() for _ in range(self.dim)]
+        _ck(lib().pmg_laplace_operator_support_points(self.h, vs[0].h, vs[1].h, vs[2].h if self.dim == 3 else None))
+        return np.stack([v.export_host() for v in vs], axis=1)
+
+    def interpolate(self, fn):
+        """A Vector of fn at the dof support points, evaluated on the host: fn(x, y, z) in 3-D, fn(x, y) in 2-D, with
+        arrays of the m coordinates; fn returns m values (or a scalar)."""
+        pts = self.support_points()
+        vals = np.broadcast_to(np.asarray(fn(*pts.T), dtype=np.float64), (len(pts),))
+        return self.vector_from(vals)
+
+    def assemble_rhs_data(self, rhs, f=None, g=None):
+        """rhs = M f_h - A_free g_D on unconstrained rows, 0 on constrained rows (pmg_laplace_operator_assemble_rhs_data)."""
+        _ck(lib().pmg_laplace_operator_assemble_rhs_data(self.h, rhs.h, f.h if f is not None else None,
+                                                         g.h if g is not None else None))
+
+    def distribute(self, u, g):
+        """u = g on the constrained dofs, other entries untouched (pmg_laplace_operator_distribute)."""
+        _ck(lib().pmg_laplace_operator_distribute(self.h, u.h, g.h))
+
 
 class _Transfer:
     def __del__(self):
