@@ -81,7 +81,10 @@ int64_t pmg_context_fused_halo_count(const pmg_context *ctx);
 
 /* ---- LaplaceOperator (include/operators/portable_laplace_operator.h:383-461) ---- */
 /* ctor (DoFHandler, AffineConstraints, overlap) :463-485.  coefficient: 0 = constant (reference),
-   1 = a(x) = 1/(0.05 + 2|x|^2) at the quadrature points (BASELINE config 5 extension). */
+   1 = a(x) = 1/(0.05 + 2|x|^2) at the quadrature points (BASELINE config 5 extension; 3-D only),
+   PMG_COEFFICIENT_CALLER = -div(a grad u) with a given by the caller at the quadrature points
+   (pmg_laplace_operator_set_coefficient; a = 1 until then).  dim 2 and 3, and _create_mapped / _create_curved. */
+#define PMG_COEFFICIENT_CALLER 2
 int pmg_laplace_operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny, int nz,
                                 unsigned dirichlet_faces, int coefficient, pmg_operator **op);
 /* The Laplace operator (with coefficient 0 or 1 as above) on a deformed structured hexahedral mesh of nx x ny x nz cells, 3-D
@@ -153,6 +156,26 @@ int pmg_laplace_operator_support_points(const pmg_operator *op, pmg_vector *x, p
 int pmg_laplace_operator_assemble_rhs_data(const pmg_operator *op, pmg_vector *rhs, const pmg_vector *f, const pmg_vector *g);
 /* u_c = g_c on every constrained dof of the stored planes, other entries untouched (AffineConstraints::distribute, :361) */
 int pmg_laplace_operator_distribute(const pmg_operator *op, pmg_vector *u, const pmg_vector *g);
+
+/* ---- coefficient from the caller: a at the QGauss(degree+1) points of the operator's cells (step-37's coefficient table,
+   FEEvaluation::quadrature_point) ----
+   The rank's quadrature-point grid: Qx = nx (degree+1) by Qy = ny (degree+1) points per q-plane, lexicographic (x fastest),
+   nqz q-planes from the global q-plane qz0 on -- the stored cell layers, the halo layer below the owned ones included.  2-D:
+   qz0 = 0, nqz = 1; a rank that holds no part of the level: nqz = 0.  Cell (cx, cy, cz), local point (a, b, m) is grid point
+   (cx (degree+1) + a, cy (degree+1) + b, cz (degree+1) + m). */
+int pmg_laplace_operator_quadrature_grid(const pmg_operator *op, int64_t *qx, int64_t *qy, int64_t *qz0, int64_t *nqz);
+/* The points of that grid: the Gauss points mapped by the cell's geometry (box, trilinear or degree-k map).  x, y, z: HOST
+   arrays of Qx Qy nqz doubles; z must be NULL in 2-D (else PMG_ERR_UNSUPPORTED).  A point two ranks store has the same
+   bits on both.  Works on every operator. */
+int pmg_laplace_operator_quadrature_points(const pmg_operator *op, double *x, double *y, double *z);
+/* Sets a at the points of pmg_laplace_operator_quadrature_points (a: HOST, Qx Qy nqz values in that order, each finite
+   and > 0; read during the call only) and recomputes the operator's per-point data and its inverse diagonal.  A second
+   call replaces the coefficient: the result equals a fresh operator given the second a.  Chebyshev smoothers keep the
+   eigenvalue estimates of the operator they were created on: create them after the coefficient is set.
+   Errors: PMG_ERR_STATE if the operator was not created with PMG_COEFFICIENT_CALLER; PMG_ERR_ARG for a == NULL or a value
+   that is not finite or <= 0, with the first offending cell and local point in pmg_last_error() (the operator is then
+   unchanged). */
+int pmg_laplace_operator_set_coefficient(pmg_operator *op, const double *a);
 
 /* ---- LinearAlgebra::distributed::Vector subset used on the path (SURVEY.md a11) ---- */
 int pmg_vector_destroy(pmg_vector *v);

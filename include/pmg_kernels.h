@@ -118,6 +118,21 @@ int pmgk_geo_rhs_f(const pmgk_level *lv, int k, const double *vert, const double
    at the degree-p Gauss-Lobatto points; x, y, z: local vectors */
 int pmgk_geo_support_points(const pmgk_level *lv, int k, const double *vert, double *x, double *y, double *z, void *stream);
 
+/* coefficient from the caller (pmg_laplace_operator_set_coefficient); a: device, one value per quadrature point in the layout
+   of coef (2-D: the (nx n1) x (ny n1) grid of the one cell layer).
+   pmgk_coef_check: err (device word, ~0 on entry) receives the smallest index i with a[i] not finite or <= 0.
+   pmgk_var_set_coef: coef = w_q a_q (a == NULL: a = 1), box levels of dim 2 and 3; gw: HOST Gauss weights on [0,1].
+   pmgk_geo_scale_coef: the six G grids *= a_q (lv->geo_stride as pmgk_geo_fill); refill them with kind 0 first.
+   pmgk_geo_quadrature_points: the mapped Gauss points (k, vert as pmgk_geo_fill, gq: HOST Gauss points on [0,1]) on the
+   quadrature-point grid of the stored cell layers, x / y / z: device, pmgk_var_coef_doubles(lv) doubles each.
+   pmgk_dim2_var_fill_dinv: inverse diagonal of a 2-D level with a coefficient (1 on constrained dofs). */
+int pmgk_coef_check(const double *a, int64_t n, unsigned long long *err, void *stream);
+int pmgk_var_set_coef(const pmgk_level *lv, const double *gw, const double *a, double *coef, void *stream);
+int pmgk_geo_scale_coef(const pmgk_level *lv, const double *a, double *geo, void *stream);
+int pmgk_geo_quadrature_points(const pmgk_level *lv, int k, const double *vert, const double *gq, double *x, double *y, double *z,
+                               void *stream);
+int pmgk_dim2_var_fill_dinv(const pmgk_level *lv, double *dinv, void *stream);
+
 /* inverse diagonal as an explicit vector (LaplaceOperator::compute_diagonal, :752-917) */
 int pmgk_fill_dinv(const pmgk_level *lv, double *dinv, void *stream);
 /* out = f * Dinv * b (first Chebyshev step from a zero guess) */

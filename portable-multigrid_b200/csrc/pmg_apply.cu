@@ -107,6 +107,9 @@ PMG_PLANE_DECL(0) PMG_PLANE_DECL(1) PMG_PLANE_DECL(2) PMG_PLANE_DECL(3) PMG_PLAN
 // 2-D levels: csrc/pmg_dim2.cu
 int pmg_dim2_apply(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out, double f1,
                    double f2, cudaStream_t s, int *geom);
+// 2-D levels with a coefficient: csrc/pmg_dim2_var.cu
+int pmg_dim2_var_apply(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out, double f1,
+                       double f2, cudaStream_t s, int *geom);
 
 // variable-coefficient levels: csrc/pmg_apply_var.cu
 int pmg_var_dispatch(const pmgk_level *lv, int mode, const double *u, const double *b, const double *xold, double *out,
@@ -133,7 +136,8 @@ static int dispatch(const pmgk_level *lv, int mode, const double *u, const doubl
   const bool chunked_kernel = lv->dim == 3 && !lv->coef &&
                               (lv->tile_variant == 1 || lv->tile_variant == 6 || (lv->tile_variant == 0 && !small_level_of(lv)));
   if (part != PMGK_PART_ALL && !chunked_kernel) return PMG_ERR_UNSUPPORTED;
-  if (lv->dim == 2) return pmg_dim2_apply(lv, mode, u, b, xold, out, f1, f2, s, geom);
+  if (lv->dim == 2) return lv->coef ? pmg_dim2_var_apply(lv, mode, u, b, xold, out, f1, f2, s, geom)
+                                    : pmg_dim2_apply(lv, mode, u, b, xold, out, f1, f2, s, geom);
   if (lv->nz < 1 || lv->cz_hi <= lv->cz_lo) return PMG_ERR_ARG;
   if (lv->coef && lv->geo_stride) return pmg_geo_dispatch(lv, mode, u, b, xold, out, f1, f2, s, geom);
   if (lv->coef) return pmg_var_dispatch(lv, mode, u, b, xold, out, f1, f2, s, geom);

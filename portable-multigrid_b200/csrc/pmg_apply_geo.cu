@@ -490,6 +490,96 @@ int geo_support_points(const pmgk_level *lv, int k, const double *vert, double *
   return 0;
 }
 
+// ---- coefficient from the caller: quadrature points, G_q scaled by a_q ------------------------------------------------
+// the mapped Gauss points of the trilinear cells (the weights of pmg_geo_point), on the quadrature-point grid of the stored
+// cell layers; one CTA row per (q-plane, q-row), threads along x.  Each point is computed from its own cell only, so a
+// point of the layer two ranks store has the same bits on both.
+template <int P>
+__global__ void k_geo_qpoints(const __grid_constant__ GeoTables t, int nx, int ny, int nqz, const double *__restrict__ vert, double *X,
+                              double *Y, double *Z)
+{
+  constexpr int N1 = P + 1;
+  const int Qx = nx * N1, Qy = ny * N1;
+  const double *s = t.a;
+  for (int row = blockIdx.x; row < Qy * nqz; row += gridDim.x) {
+    const int qy = row % Qy, lqz = row / Qy;
+    const int cy = qy / N1, b = qy % N1, lcz = lqz / N1, m = lqz % N1;
+    for (int qx = threadIdx.x; qx < Qx; qx += blockDim.x) {
+      const int cx = qx / N1, a = qx % N1;
+      double v[8][3];
+      geo_load_cell(vert, nx, ny, cx, cy, lcz, v);
+      const double L[2][3] = {{1.0 - s[a], 1.0 - s[b], 1.0 - s[m]}, {s[a], s[b], s[m]}};
+      double x[3] = {0.0, 0.0, 0.0};
+      for (int c = 0; c < 8; ++c) {
+        const double w = L[c & 1][0] * L[c >> 1 & 1][1] * L[c >> 2][2];
+        for (int d = 0; d < 3; ++d) x[d] += w * v[c][d];
+      }
+      const int64_t o = (int64_t)row * Qx + qx;
+      X[o] = x[0];
+      Y[o] = x[1];
+      Z[o] = x[2];
+    }
+  }
+}
+
+// as k_geo_qpoints for curved cells: the degree-k map (pmg_curved_map) with the tables t at the Gauss points
+template <int P>
+__global__ void k_curved_qpoints(const __grid_constant__ CurvedTables t, int k, int nx, int ny, int nqz, const double *__restrict__ nodes,
+                                 double *X, double *Y, double *Z)
+{
+  constexpr int N1 = P + 1;
+  const int Qx = nx * N1, Qy = ny * N1, k1 = k + 1;
+  const int64_t sy = (int64_t)nx * k + 1, sz = sy * ((int64_t)ny * k + 1);
+  for (int row = blockIdx.x; row < Qy * nqz; row += gridDim.x) {
+    const int qy = row % Qy, lqz = row / Qy;
+    const int cy = qy / N1, b = qy % N1, lcz = lqz / N1, m = lqz % N1;
+    for (int qx = threadIdx.x; qx < Qx; qx += blockDim.x) {
+      const int cx = qx / N1, a = qx % N1;
+      double x[3], J[3][3];
+      pmg_curved_map(curved_cell_node(nodes, nx, ny, k, cx, cy, lcz), sy, sz, k, t.L + a * k1, t.dL + a * k1, t.L + b * k1,
+                     t.dL + b * k1, t.L + m * k1, t.dL + m * k1, x, J);
+      const int64_t o = (int64_t)row * Qx + qx;
+      X[o] = x[0];
+      Y[o] = x[1];
+      Z[o] = x[2];
+    }
+  }
+}
+
+// G_q *= a_q, the six grids of the stored cell layers (a: one grid of that layout)
+__global__ void k_geo_scale_coef(const double *__restrict__ a, int64_t n, int64_t gstride, double *geo)
+{
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const double ai = a[i];
+    for (int e = 0; e < 6; ++e) geo[i + e * gstride] *= ai;
+  }
+}
+
+template <int P>
+int geo_quadrature_points(const pmgk_level *lv, int k, const double *vert, const double *gq, double *x, double *y, double *z,
+                          cudaStream_t s)
+{
+  constexpr int N1 = P + 1;
+  const int Qx = lv->nx * N1, Qy = lv->ny * N1, nqz = (lv->cz_hi - lv->coef_cz0) * N1;
+  if (nqz <= 0) return 0;
+  int64_t rows = (int64_t)Qy * nqz;
+  const int64_t cap = (int64_t)pmgk_device_sm_count() * 32;
+  if (rows > cap) rows = cap;
+  if (k == 1) {
+    GeoTables t;
+    for (int i = 0; i < N1; ++i) t.a[i] = gq[i];
+    k_geo_qpoints<P><<<(unsigned)rows, pmg_var_row_threads(Qx), 0, s>>>(t, lv->nx, lv->ny, nqz, vert, x, y, z);
+  } else {
+    CurvedTables t;
+    double unused_w[N1] = {};
+    curved_tables(k, N1, gq, unused_w, t);
+    k_curved_qpoints<P><<<(unsigned)rows, pmg_var_row_threads(Qx), 0, s>>>(t, k, lv->nx, lv->ny, nqz, vert, x, y, z);
+  }
+  PMG_CUDA_CHECK(cudaGetLastError());
+  pmg_count_launch(1);
+  return 0;
+}
+
 template <int P>
 int fill_geo(const pmgk_level *lv, int k, int c5, const double *vert, const double *gq, const double *gw, double *geo,
              unsigned long long *err, cudaStream_t s)
@@ -698,4 +788,32 @@ extern "C" int pmgk_geo_fill_dinv(const pmgk_level *lv, const double *S2, const 
 #undef PMG_GEO_CASE
     default: return PMG_ERR_UNSUPPORTED;
   }
+}
+
+extern "C" int pmgk_geo_quadrature_points(const pmgk_level *lv, int k, const double *vert, const double *gq, double *x, double *y,
+                                          double *z, void *stream)
+{
+  if (!lv || !vert || !gq || !x || !y || !z) return PMG_ERR_ARG;
+  if (k < 1 || k >= PMGK_MAX_N1) return PMG_ERR_UNSUPPORTED;
+  switch (lv->degree) {
+#define PMG_GEO_CASE(P, BX, BY, MINB) \
+  case P: return geo_quadrature_points<P>(lv, k, vert, gq, x, y, z, (cudaStream_t)stream);
+#include "pmg_apply_geo_tiles.inc"
+#undef PMG_GEO_CASE
+    default: return PMG_ERR_UNSUPPORTED;
+  }
+}
+
+extern "C" int pmgk_geo_scale_coef(const pmgk_level *lv, const double *a, double *geo, void *stream)
+{
+  if (!lv || !a || !geo || lv->geo_stride != pmgk_var_coef_doubles(lv)) return PMG_ERR_ARG;
+  const int64_t n = lv->geo_stride;
+  if (n == 0) return 0;
+  int64_t blocks = (n + 255) / 256;
+  const int64_t cap = (int64_t)pmgk_device_sm_count() * 16;
+  if (blocks > cap) blocks = cap;
+  k_geo_scale_coef<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, n, lv->geo_stride, geo);
+  PMG_CUDA_CHECK(cudaGetLastError());
+  pmg_count_launch(1);
+  return 0;
 }

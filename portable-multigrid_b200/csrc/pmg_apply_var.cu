@@ -152,6 +152,46 @@ int fill_dinv(const pmgk_level *lv, const double *S2, const double *G2, double *
   return 0;
 }
 
+// ---- coefficient from the caller (pmg_laplace_operator_set_coefficient) ------------------------------------------------
+// err = the smallest index i with a[i] not finite or <= 0 (err is ~0 on entry)
+__global__ void k_coef_check(const double *__restrict__ a, int64_t n, unsigned long long *err)
+{
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    if (!(isfinite(a[i]) && a[i] > 0.0)) atomicMin(err, (unsigned long long)i);
+}
+
+// W = w_q a_q on the quadrature-point grid of the stored cell layers (a == NULL: a = 1); wz: 1 = the weight of the q-plane
+// enters (3-D), 0 = one plane of the 2-D grid
+template <int P>
+__global__ void k_var_coef_caller(const __grid_constant__ VarTables t, int Qx, int Qy, int nqz, int wz, const double *__restrict__ a,
+                                  double *coef)
+{
+  constexpr int N1 = P + 1;
+  for (int row = blockIdx.x; row < Qy * nqz; row += gridDim.x) {
+    const int qy = row % Qy, qz = row / Qy;
+    const double wyz = t.b[qy % N1] * (wz ? t.b[qz % N1] : 1.0);
+    const int64_t o = (int64_t)row * Qx;
+    for (int qx = threadIdx.x; qx < Qx; qx += blockDim.x) coef[o + qx] = t.b[qx % N1] * wyz * (a ? a[o + qx] : 1.0);
+  }
+}
+
+template <int P>
+int set_coef(const pmgk_level *lv, const double *gw, const double *a, double *coef, cudaStream_t s)
+{
+  constexpr int N1 = P + 1;
+  VarTables t;
+  for (int i = 0; i < N1; ++i) { t.a[i] = 0.0; t.b[i] = gw[i]; }
+  const int Qx = lv->nx * N1, Qy = lv->ny * N1, nqz = lv->dim == 2 ? 1 : (lv->cz_hi - lv->coef_cz0) * N1;
+  if (nqz <= 0) return 0;
+  int64_t rows = (int64_t)Qy * nqz;
+  const int64_t cap = (int64_t)pmgk_device_sm_count() * 32;
+  if (rows > cap) rows = cap;
+  k_var_coef_caller<P><<<(unsigned)rows, pmg_var_row_threads(Qx), 0, s>>>(t, Qx, Qy, nqz, lv->dim == 3, a, coef);
+  PMG_CUDA_CHECK(cudaGetLastError());
+  pmg_count_launch(1);
+  return 0;
+}
+
 } // namespace
 
 // called by pmgk_apply (pmg_apply.cu) for levels that carry a coefficient
@@ -207,6 +247,36 @@ extern "C" int pmgk_var_fill_dinv(const pmgk_level *lv, const double *S2, const 
     case 7: return fill_dinv<7>(lv, S2, G2, dinv, (cudaStream_t)stream);
     case 8: return fill_dinv<8>(lv, S2, G2, dinv, (cudaStream_t)stream);
     case 9: return fill_dinv<9>(lv, S2, G2, dinv, (cudaStream_t)stream);
+    default: return PMG_ERR_UNSUPPORTED;
+  }
+}
+
+extern "C" int pmgk_coef_check(const double *a, int64_t n, unsigned long long *err, void *stream)
+{
+  if (!a || !err || n < 0) return PMG_ERR_ARG;
+  if (n == 0) return 0;
+  int64_t blocks = (n + 255) / 256;
+  const int64_t cap = (int64_t)pmgk_device_sm_count() * 16;
+  if (blocks > cap) blocks = cap;
+  k_coef_check<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, n, err);
+  PMG_CUDA_CHECK(cudaGetLastError());
+  pmg_count_launch(1);
+  return 0;
+}
+
+extern "C" int pmgk_var_set_coef(const pmgk_level *lv, const double *gw, const double *a, double *coef, void *stream)
+{
+  if (!lv || !gw || !coef) return PMG_ERR_ARG;
+  switch (lv->degree) {
+    case 1: return set_coef<1>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 2: return set_coef<2>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 3: return set_coef<3>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 4: return set_coef<4>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 5: return set_coef<5>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 6: return set_coef<6>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 7: return set_coef<7>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 8: return set_coef<8>(lv, gw, a, coef, (cudaStream_t)stream);
+    case 9: return set_coef<9>(lv, gw, a, coef, (cudaStream_t)stream);
     default: return PMG_ERR_UNSUPPORTED;
   }
 }

@@ -99,7 +99,10 @@ static double arg_double(int argc, char **argv, const char *name, double def)
    ||u||_L2 = 0.14143644722133), --mapping-degree K the geometry degree of the cells of --distort / --shell: 1 (default)
    trilinear cells, 0 the level's FE degree (MappingQ(p) on every level), K >= 2 curved cells of degree K,
    --manufactured 1 solves -div(grad u) = f, u = g on the Dirichlet faces, for a known smooth u* (manufactured_values) with f
-   and g = u* interpolated at the dof support points, and prints ||u_h - I_h u*||_L2 after the solution norm */
+   and g = u* interpolated at the dof support points, and prints ||u_h - I_h u*||_L2 after the solution norm,
+   --coefficient 2 solves -div(a grad u) = 1 with a jump coefficient given through PMG_COEFFICIENT_CALLER on every level at
+   the level's own quadrature points: a = 100 in [1/4, 3/4]^dim and 1 elsewhere (cube / square), a = 100 for r < 1.5 and 1
+   elsewhere (--shell 1) */
 static int g_coefficient = 0, g_profile = 0, g_dim = 3, g_shell = 0, g_mapping_degree = 1, g_manufactured = 0;
 static double g_tol = 1e-12, g_distort = 0.0;
 static void common_options(int argc, char **argv)
@@ -164,10 +167,34 @@ static int manufactured_rhs(pmg_operator *A, pmg_vector *rhs, pmg_vector *ustar)
   return rc;
 }
 
+/* --coefficient 2: the jump coefficient at the operator's quadrature points (pmg_laplace_operator_set_coefficient) */
+static double jump_coefficient(double x, double y, double z)
+{
+  if (g_shell) return sqrt(x * x + y * y) < 1.5 ? 100.0 : 1.0;
+  const int inside = x >= 0.25 && x <= 0.75 && y >= 0.25 && y <= 0.75 && (g_dim == 2 || (z >= 0.25 && z <= 0.75));
+  return inside ? 100.0 : 1.0;
+}
+
+static int set_jump_coefficient(pmg_operator *op)
+{
+  int64_t qx = 0, qy = 0, qz0 = 0, nqz = 0;
+  int rc = pmg_laplace_operator_quadrature_grid(op, &qx, &qy, &qz0, &nqz);
+  const size_t n = (size_t)(qx * qy * nqz);
+  if (rc != PMG_OK || n == 0) return rc;
+  double *h = (double *)malloc(sizeof(double) * 4 * n);
+  if (!h) return PMG_ERR_NOMEM;
+  double *x = h, *y = h + n, *z = h + 2 * n, *a = h + 3 * n;
+  rc = pmg_laplace_operator_quadrature_points(op, x, y, g_dim == 3 ? z : NULL);
+  for (size_t i = 0; i < n && rc == PMG_OK; ++i) a[i] = jump_coefficient(x[i], y[i], g_dim == 3 ? z[i] : 0.0);
+  if (rc == PMG_OK) rc = pmg_laplace_operator_set_coefficient(op, a);
+  free(h);
+  return rc;
+}
+
 /* the level's operator: on the unit cube, or with --distort / --shell on the image of the unit cube's mesh of n^3 cells
    under the map, with cells of geometry degree k: the map evaluated at the degree-k Gauss-Lobatto grid of every cell
    (pmg_laplace_operator_create_curved; k = 1 gives the vertices of the trilinear cells, nested on the h-levels) */
-static int create_level_operator(pmg_context *ctx, const level_t *lv, pmg_operator **op)
+static int create_level_operator_geometry(pmg_context *ctx, const level_t *lv, pmg_operator **op)
 {
   if (g_distort == 0.0 && !g_shell)
     return pmg_laplace_operator_create(ctx, g_dim, lv->degree, lv->n, lv->n, lv->n, PMG_ALL_FACES, g_coefficient, op);
@@ -209,6 +236,13 @@ static int create_level_operator(pmg_context *ctx, const level_t *lv, pmg_operat
   return rc;
 }
 
+static int create_level_operator(pmg_context *ctx, const level_t *lv, pmg_operator **op)
+{
+  int rc = create_level_operator_geometry(ctx, lv, op);
+  if (rc == PMG_OK && g_coefficient == PMG_COEFFICIENT_CALLER) rc = set_jump_coefficient(*op);
+  return rc;
+}
+
 static long long n_dofs_of(int degree, int n)
 {
   long long r = 1;
@@ -223,6 +257,9 @@ static int solve_hierarchy(pmg_context *ctx, const level_t *lv, int L, int pre, 
   pmg_transfer *tr[MAXL];
   pmg_chebyshev *sm[MAXL];
   memset(tr, 0, sizeof(tr));
+  if (g_coefficient == PMG_COEFFICIENT_CALLER)
+    RPRINT("  coefficient: a = 100 %s, 1 elsewhere (given at every level's quadrature points)\n",
+           g_shell ? "for r < 1.5" : (g_dim == 2 ? "in [1/4, 3/4]^2" : "in [1/4, 3/4]^3"));
   if (g_shell) RPRINT("  curved mesh: quarter cylindrical shell 1 <= r <= 2, 0 <= theta <= pi/2, 0 <= z <= 1\n");
   else if (g_distort != 0.0) RPRINT("  mapped mesh: x + %g sin(pi x) sin(pi y) sin(pi z) (1, 1, 1)\n", g_distort);
   if ((g_shell || g_distort != 0.0) && g_mapping_degree != 1) {

@@ -6,7 +6,7 @@
  * Defaults = the reference program (:439-441, :399): dim = 2, fe_degree = 7, mg_levels = 7, seven refinement cycles
  * (1 .. 64^2 cells).  --dim 3 runs the same hierarchy on the unit cube (then think of --degree 4 --cycles 5).
  * --hp 1 selects BASELINE config 2 instead: p = 4 -> 2 -> 1 followed by geometric levels.
- * --coefficient 1, --tol T, --profile 1, --distort EPS, --shell 1, --mapping-degree K: see driver_common.h (BASELINE config 5: --hp 1 --degree 5
+ * --coefficient 1 | 2, --tol T, --profile 1, --distort EPS, --shell 1, --mapping-degree K: see driver_common.h (BASELINE config 5: --hp 1 --degree 5
  * --coefficient 1 --tol 1e-10).
  */
 #include "driver_common.h"

@@ -17,6 +17,7 @@
    (csrc/pmg_apply_var.h); the inverse diagonal of such an operator is an explicit vector. */
 static int var_diagonal(pmg_operator *op)
 {
+  if (op->dim == 2) return pmgk_dim2_var_fill_dinv(&op->lv, op->dinv->d, op->ctx->stream);
   const int n1 = op->degree + 1;
   double Sq[PMGK_MAX_N1 * PMGK_MAX_N1], G[PMGK_MAX_N1 * PMGK_MAX_N1];
   pmg_fe_shape_tables(op->degree, Sq, NULL, G, NULL, NULL);
@@ -24,6 +25,17 @@ static int var_diagonal(pmg_operator *op)
   return pmgk_var_fill_dinv(&op->lv, Sq, G, op->dinv->d, op->ctx->stream);
 }
 
+/* values of the coefficient the operator stores: one per quadrature point of the stored cell layers (3-D: the layout of
+   pmgk_var_coef_doubles, 2-D: the (nx n1) x (ny n1) grid of the one cell layer) */
+static int64_t quadrature_count(const pmg_operator *op)
+{
+  if (!op->lay.active) return 0;
+  if (op->dim == 2) return (int64_t)op->lv.nx * (op->degree + 1) * op->lv.ny * (op->degree + 1);
+  return pmgk_var_coef_doubles(&op->lv);
+}
+
+/* coefficient 1: the C5 coefficient; PMG_COEFFICIENT_CALLER: a = 1 until pmg_laplace_operator_set_coefficient.  A 2-D
+   level stores two more grids of the same size behind w_q a_q: the scratch of its two-pass apply (csrc/pmg_dim2_var.h). */
 static int setup_coefficient(pmg_operator *op)
 {
   pmgk_level *lv = &op->lv;
@@ -32,12 +44,13 @@ static int setup_coefficient(pmg_operator *op)
   lv->coef_cz0 = lv->z0 / op->degree;
   PMG_CHECK(pmg_vector_create_layout(op->ctx, &op->lay, &op->dinv));
   if (!op->lay.active) return PMG_OK;
-  const int64_t n = pmgk_var_coef_doubles(lv);
+  const int64_t n = quadrature_count(op) * (op->dim == 2 ? 3 : 1);
   if (cudaMalloc((void **)&op->d_coef, sizeof(double) * (size_t)n) != cudaSuccess) {
     pmg_set_error("cudaMalloc of %lld coefficient values failed", (long long)n);
     return PMG_ERR_NOMEM;
   }
-  PMG_CHECK(pmgk_var_fill_coef(lv, op->coefficient, gq, gw, op->d_coef, op->ctx->stream));
+  if (op->coefficient == PMG_COEFFICIENT_CALLER) PMG_CHECK(pmgk_var_set_coef(lv, gw, NULL, op->d_coef, op->ctx->stream));
+  else PMG_CHECK(pmgk_var_fill_coef(lv, op->coefficient, gq, gw, op->d_coef, op->ctx->stream));
   lv->coef = op->d_coef;
   PMG_CHECK(var_diagonal(op));
   lv->dinv_vec = op->dinv->d;
@@ -87,7 +100,8 @@ static int setup_geometry(pmg_operator *op, const double *nodes)
   d_err = (unsigned long long *)(op->d_vert + nv);
   if (cudaMemcpyAsync(op->d_vert, nodes + vplane * k * lv->coef_cz0, sizeof(double) * nv, cudaMemcpyHostToDevice, st) != cudaSuccess ||
       cudaMemsetAsync(d_err, 0xFF, sizeof(unsigned long long), st) != cudaSuccess) rc = PMG_ERR_CUDA;
-  if (rc == PMG_OK) rc = pmgk_geo_fill(lv, k, op->coefficient, op->d_vert, gq, gw, op->d_coef, d_err, st);
+  /* PMG_COEFFICIENT_CALLER: a = 1 until pmg_laplace_operator_set_coefficient scales the grids */
+  if (rc == PMG_OK) rc = pmgk_geo_fill(lv, k, op->coefficient == 1, op->d_vert, gq, gw, op->d_coef, d_err, st);
   if (rc == PMG_OK && cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
   if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* nodes and h_err are pageable */
   if (rc != PMG_OK) return rc;
@@ -109,9 +123,12 @@ static int operator_create(pmg_context *ctx, int dim, int degree, int nx, int ny
   if (!ctx || !out || nx < 1 || ny < 1 || nz < 1) { pmg_set_error("operator_create: bad arguments"); return PMG_ERR_ARG; }
   if (dim != 2 && dim != 3) { pmg_set_error("dim = %d: the reference instantiates dim = 2 and dim = 3", dim); return PMG_ERR_UNSUPPORTED; }
   if (dim == 2) { nz = 1; faces &= 0xFu; }
-  if (dim == 2 && coefficient != 0) { pmg_set_error("the variable-coefficient operator is 3-D only"); return PMG_ERR_UNSUPPORTED; }
+  if (dim == 2 && coefficient == 1) { pmg_set_error("the coefficient 1/(0.05 + 2|x|^2) is 3-D only"); return PMG_ERR_UNSUPPORTED; }
   if (degree < 1 || degree > PMG_MAX_DEGREE) { pmg_set_error("degree %d outside 1..%d", degree, PMG_MAX_DEGREE); return PMG_ERR_UNSUPPORTED; }
-  if (coefficient != 0 && coefficient != 1) { pmg_set_error("coefficient %d: 0 = constant, 1 = 1/(0.05 + 2|x|^2)", coefficient); return PMG_ERR_UNSUPPORTED; }
+  if (coefficient != 0 && coefficient != 1 && coefficient != PMG_COEFFICIENT_CALLER) {
+    pmg_set_error("coefficient %d: 0 = constant, 1 = 1/(0.05 + 2|x|^2), %d = given by the caller", coefficient, PMG_COEFFICIENT_CALLER);
+    return PMG_ERR_UNSUPPORTED;
+  }
   if ((int64_t)(nx * (int64_t)degree + 1) * (ny * (int64_t)degree + 1) >= (int64_t)1 << 31) return PMG_ERR_ARG;
   pmg_operator *op = (pmg_operator *)calloc(1, sizeof(*op));
   if (!op) return PMG_ERR_NOMEM;
@@ -654,4 +671,125 @@ int pmg_laplace_operator_distribute(const pmg_operator *op, pmg_vector *u, const
   PMG_CHECK(pmg_enter(op->ctx));
   if (!op->lay.active || u == g) return PMG_OK;
   return pmgk_constrained_copy(&op->lv, u->d, g->d, 0, op->ctx->stream);
+}
+
+/* ---- coefficient from the caller (PMG_COEFFICIENT_CALLER) ----------------------------------------------------------------- */
+int pmg_laplace_operator_quadrature_grid(const pmg_operator *op, int64_t *qx, int64_t *qy, int64_t *qz0, int64_t *nqz)
+{
+  if (!op) return PMG_ERR_ARG;
+  const int n1 = op->degree + 1;
+  const int64_t Q = quadrature_count(op), plane = (int64_t)op->lay.nx * n1 * op->lay.ny * n1;
+  if (qx) *qx = (int64_t)op->lay.nx * n1;
+  if (qy) *qy = (int64_t)op->lay.ny * n1;
+  if (qz0) *qz0 = op->dim == 2 ? 0 : (int64_t)(op->lay.z0 / op->degree) * n1;
+  if (nqz) *nqz = Q / plane;
+  return PMG_OK;
+}
+
+/* Box: the Gauss points (c + g_a) h of every direction as three outer products of 1-D lines with ones (pmgk_outer3, exact);
+   mapped: the cells' maps at the Gauss points on the device. */
+int pmg_laplace_operator_quadrature_points(const pmg_operator *op, double *x, double *y, double *z)
+{
+  if (!op || !x || !y) return PMG_ERR_ARG;
+  if (op->dim == 2 && z) { pmg_set_error("quadrature_points: the 2-D operator has no z coordinate (pass z = NULL)"); return PMG_ERR_UNSUPPORTED; }
+  if (op->dim == 3 && !z) return PMG_ERR_ARG;
+  PMG_CHECK(pmg_enter(op->ctx));
+  const int64_t n = quadrature_count(op);
+  if (n == 0) return PMG_OK;
+  const int n1 = op->degree + 1;
+  int64_t Qx, Qy, qz0, nqz;
+  PMG_CHECK(pmg_laplace_operator_quadrature_grid(op, &Qx, &Qy, &qz0, &nqz));
+  double gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
+  pmg_fe_gauss(n1, gq, gw);
+  cudaStream_t st = op->ctx->stream;
+  const int nout = op->dim;
+  const int64_t nmax = Qx > Qy ? (Qx > nqz ? Qx : nqz) : (Qy > nqz ? Qy : nqz);
+  const size_t nl = (size_t)(Qx + Qy + nqz + nmax);
+  double *d = NULL, *h = (double *)malloc(sizeof(double) * nl);
+  if (!h) return PMG_ERR_NOMEM;
+  int rc = PMG_OK;
+  if (cudaMallocAsync((void **)&d, sizeof(double) * ((size_t)nout * n + nl), st) != cudaSuccess) { free(h); return PMG_ERR_NOMEM; }
+  double *dx = d, *dy = d + n, *dz = op->dim == 3 ? d + 2 * n : NULL;
+  if (op->mapped) {
+    rc = pmgk_geo_quadrature_points(&op->lv, op->geo_degree, op->d_vert, gq, dx, dy, dz, st);
+  } else {
+    /* host: the lines x, y, z (global q-planes qz0 ..), then ones */
+    const int64_t N[3] = {Qx, Qy, nqz};
+    double *line[3] = {h, h + Qx, h + Qx + Qy}, *ones = h + Qx + Qy + nqz;
+    for (int e = 0; e < 3; ++e)
+      for (int64_t q = 0; q < N[e]; ++q) {
+        const int64_t g = q + (e == 2 ? qz0 : 0);
+        line[e][q] = (e == 2 && op->dim == 2) ? 0.0 : (double)((g / n1) + gq[g % n1]) * op->lv.h[e];
+      }
+    for (int64_t i = 0; i < nmax; ++i) ones[i] = 1.0;
+    double *dl = d + (size_t)nout * n, *d1 = dl + Qx + Qy + nqz;
+    if (cudaMemcpyAsync(dl, h, sizeof(double) * nl, cudaMemcpyHostToDevice, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+    if (rc == PMG_OK) rc = pmgk_outer3(dx, dl, d1, d1, (int)Qx, (int)Qy, (int)nqz, st);
+    if (rc == PMG_OK) rc = pmgk_outer3(dy, d1, dl + Qx, d1, (int)Qx, (int)Qy, (int)nqz, st);
+    if (rc == PMG_OK && dz) rc = pmgk_outer3(dz, d1, d1, dl + Qx + Qy, (int)Qx, (int)Qy, (int)nqz, st);
+  }
+  if (rc == PMG_OK && cudaMemcpyAsync(x, dx, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (rc == PMG_OK && cudaMemcpyAsync(y, dy, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (rc == PMG_OK && dz && cudaMemcpyAsync(z, dz, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  cudaFreeAsync(d, st);
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* h, x, y, z are pageable */
+  free(h);
+  return rc;
+}
+
+/* a: HOST, one value per quadrature point in the order of pmg_laplace_operator_quadrature_points.  The values are uploaded
+   and checked on the device before anything of the operator changes; then box levels refill w_q a_q, mapped levels refill
+   their G grids with a = 1 from the kept nodes and scale them by a_q (so a second call replaces, never compounds), and the
+   inverse diagonal is recomputed. */
+int pmg_laplace_operator_set_coefficient(pmg_operator *op, const double *a)
+{
+  if (!op) return PMG_ERR_ARG;
+  if (op->coefficient != PMG_COEFFICIENT_CALLER) {
+    pmg_set_error("set_coefficient: the operator was created with coefficient %d, not PMG_COEFFICIENT_CALLER", op->coefficient);
+    return PMG_ERR_STATE;
+  }
+  if (!a) { pmg_set_error("set_coefficient: no values"); return PMG_ERR_ARG; }
+  PMG_CHECK(pmg_enter(op->ctx));
+  const int64_t n = quadrature_count(op);
+  if (n == 0) return PMG_OK;
+  pmgk_level *lv = &op->lv;
+  cudaStream_t st = op->ctx->stream;
+  double *d_a = NULL;
+  unsigned long long h_err = ~0ull, *d_err;
+  if (cudaMallocAsync((void **)&d_a, sizeof(double) * (size_t)n + sizeof(unsigned long long), st) != cudaSuccess) return PMG_ERR_NOMEM;
+  d_err = (unsigned long long *)(d_a + n);
+  int rc = PMG_OK;
+  if (cudaMemcpyAsync(d_a, a, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+      cudaMemsetAsync(d_err, 0xFF, sizeof(unsigned long long), st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (rc == PMG_OK) rc = pmgk_coef_check(d_a, n, d_err, st);
+  if (rc == PMG_OK && cudaMemcpyAsync(&h_err, d_err, sizeof(h_err), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = PMG_ERR_CUDA;
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == PMG_OK) rc = PMG_ERR_CUDA; /* a and h_err are pageable */
+  if (rc == PMG_OK && h_err != ~0ull) {
+    const int n1 = op->degree + 1;
+    const long long i = (long long)h_err, Qx = (long long)lv->nx * n1, Qy = (long long)lv->ny * n1;
+    const long long qx = i % Qx, qy = i / Qx % Qy, qz = i / (Qx * Qy) + (op->dim == 2 ? 0 : (long long)lv->coef_cz0 * n1);
+    if (op->dim == 2)
+      pmg_set_error("set_coefficient: a = %g at value %lld: cell (%lld, %lld), local point (%lld, %lld); a must be finite and > 0",
+                    a[i], i, qx / n1, qy / n1, qx % n1, qy % n1);
+    else
+      pmg_set_error("set_coefficient: a = %g at value %lld: cell (%lld, %lld, %lld), local point (%lld, %lld, %lld); a must be finite "
+                    "and > 0", a[i], i, qx / n1, qy / n1, qz / n1, qx % n1, qy % n1, qz % n1);
+    rc = PMG_ERR_ARG;
+  }
+  if (rc == PMG_OK && op->mapped) {
+    double gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
+    pmg_fe_gauss(op->degree + 1, gq, gw);
+    /* the nodes were validated at creation: the error word is reset and not read */
+    if (cudaMemsetAsync(d_err, 0xFF, sizeof(unsigned long long), st) != cudaSuccess) rc = PMG_ERR_CUDA;
+    if (rc == PMG_OK) rc = pmgk_geo_fill(lv, op->geo_degree, 0, op->d_vert, gq, gw, op->d_coef, d_err, st);
+    if (rc == PMG_OK) rc = pmgk_geo_scale_coef(lv, d_a, op->d_coef, st);
+    if (rc == PMG_OK) rc = geo_diagonal(op);
+  } else if (rc == PMG_OK) {
+    double gq[PMGK_MAX_N1], gw[PMGK_MAX_N1];
+    pmg_fe_gauss(op->degree + 1, gq, gw);
+    rc = pmgk_var_set_coef(lv, gw, d_a, op->d_coef, st);
+    if (rc == PMG_OK) rc = var_diagonal(op);
+  }
+  cudaFreeAsync(d_a, st);
+  return rc;
 }

@@ -16,6 +16,7 @@ LIB_PATH = os.path.normpath(os.path.join(_HERE, "..", "..", "lib", "libpmg.so"))
 PMG_ALL_FACES = 0x3F
 PMG_INVALID_DEGREE = -1
 PMG_MAX_DEGREE = 9
+PMG_COEFFICIENT_CALLER = 2
 _dp = C.POINTER(C.c_double)
 _vp = C.c_void_p
 
@@ -226,7 +227,18 @@ class LaplaceOperator:
         structured mesh, shape (nz+1, ny+1, nx+1, 3) or flat in that order (pmg_laplace_operator_create_mapped); 3-D only.
         nodes: instead of vertices, the (nx k+1)(ny k+1)(nz k+1) geometry support points of curved cells of degree
         k = geometry_degree (mesh_nodes; pmg_laplace_operator_create_curved), shape (nz k+1, ny k+1, nx k+1, 3) or flat;
-        geometry_degree None: the k the array's size implies."""
+        geometry_degree None: the k the array's size implies.
+        coefficient: 0 (a = 1), 1 (a = 1/(0.05 + 2|x|^2), 3-D), PMG_COEFFICIENT_CALLER (a = 1 until set_coefficient) or a
+        callable fn(x, y[, z]) -> a: the operator is created with PMG_COEFFICIENT_CALLER and given fn at its
+        quadrature_points()."""
+        fn = coefficient if callable(coefficient) else None
+        if fn is not None:
+            coefficient = PMG_COEFFICIENT_CALLER
+        self._create(ctx, degree, n, dirichlet_faces, dim, coefficient, vertices, nodes, geometry_degree)
+        if fn is not None:
+            self.set_coefficient(self.evaluate_at_quadrature_points(fn))
+
+    def _create(self, ctx, degree, n, dirichlet_faces, dim, coefficient, vertices, nodes, geometry_degree):
         if isinstance(n, int):
             n = (n,) * dim
         n = tuple(n) + (1,) * (3 - len(n))  # dim = 2: (nx, ny); the C-ABI ignores nz
@@ -347,6 +359,35 @@ class LaplaceOperator:
         """u = g on the constrained dofs, other entries untouched (pmg_laplace_operator_distribute)."""
         _ck(lib().pmg_laplace_operator_distribute(self.h, u.h, g.h))
 
+    def quadrature_grid(self):
+        """(Qx, Qy, qz0, nqz): this rank's quadrature-point grid (pmg_laplace_operator_quadrature_grid)."""
+        v = [C.c_int64() for _ in range(4)]
+        _ck(lib().pmg_laplace_operator_quadrature_grid(self.h, *[C.byref(x) for x in v]))
+        return tuple(x.value for x in v)
+
+    def quadrature_points(self):
+        """The QGauss(p+1) points of the rank's stored cells, an (n, dim) array in the order set_coefficient takes
+        (pmg_laplace_operator_quadrature_points)."""
+        qx, qy, _, nqz = self.quadrature_grid()
+        xs = [np.empty(qx * qy * nqz) for _ in range(self.dim)]
+        _ck(lib().pmg_laplace_operator_quadrature_points(self.h, _np_ptr(xs[0]), _np_ptr(xs[1]),
+                                                         _np_ptr(xs[2]) if self.dim == 3 else None))
+        return np.stack(xs, axis=1)
+
+    def evaluate_at_quadrature_points(self, fn):
+        """fn(x, y[, z]) at quadrature_points(), broadcast to one value per point."""
+        pts = self.quadrature_points()
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(fn(*pts.T), dtype=np.float64), (len(pts),)))
+
+    def set_coefficient(self, values):
+        """a at quadrature_points(), one finite positive value per point (pmg_laplace_operator_set_coefficient); create the
+        Chebyshev smoothers of the operator afterwards."""
+        a = np.ascontiguousarray(values, dtype=np.float64).reshape(-1)
+        qx, qy, _, nqz = self.quadrature_grid()
+        if a.size != qx * qy * nqz:
+            raise PmgError(-1, "set_coefficient: %d values for %d quadrature points" % (a.size, qx * qy * nqz))
+        _ck(lib().pmg_laplace_operator_set_coefficient(self.h, _np_ptr(a)))
+
 
 class _Transfer:
     def __del__(self):
@@ -466,7 +507,8 @@ def build_hierarchy(ctx, levels, pre=2, post=2, degree=5, smoothing_range=15.0, 
     """levels: list of (degree, n_cells) coarse -> fine; consecutive levels must be related by one
     global refinement (h) or a degree change on the same mesh (p).  Smoother parameters as in the
     reference drivers (program.cc:267-279).  coefficient = 1: every level discretises -div(a grad u) with
-    a = 1/(0.05 + 2|x|^2) at its own quadrature points (BASELINE config 5).  vertices: the finest mesh's vertices
+    a = 1/(0.05 + 2|x|^2) at its own quadrature points (BASELINE config 5); a callable fn(x, y[, z]): every level is given
+    fn at its own quadrature points (step-37's coefficient table on every level), before its smoother is created.  vertices: the finest mesh's vertices
     (LaplaceOperator); a coarser mesh takes every 2^k-th vertex in each direction (nested meshes), p-levels share them.
     mapping: instead of vertices, a map of the unit cube (mesh_nodes); every level gets curved cells interpolating it,
     of the level's FE degree (MappingQ(p) on every level) or of geometry_degree when that is given."""
